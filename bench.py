@@ -9,9 +9,11 @@ the k-NN kernel; `--exchange nccl` = all-gather + merge kernel).  A "step" is on
 query batch against the whole database.  `value` is whole-job Gpairs/s with the database and the
 query already resident in HBM; `e2e` is the same metric through the reference-facing drop-in
 (`ShardedKeyframeDatabase.knnMatch`, the cv2 collection API `bf.add(...); bf.knnMatch(q, k=2)`)
-with the query in host memory and DMatch tuples out.
+with the query in host memory and DMatch tuples out.  `--dump-outputs DIR` writes the result of the last
+timed step (imgIdx, trainIdx, distance of the two nearest rows per query) as .npy files; the inputs are
+seeded, so two builds run with the same arguments can be compared file for file.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     torchrun --nproc-per-node N bench.py --gpus N ...
 
 Other workloads (--workload c1|c2|c3|c5) are single-GPU lines used for DESIGN.md / profiles.
@@ -331,7 +333,7 @@ def tensor_roofline(nat, peaks, peak_src, variant_used, nq, nt_local, kern_ms, b
 
 
 def time_c4(db, q_dev, steps, warmup, barrier, nat, torch, local_rank):
-    """K timed steps, inputs resident: (ms per step, mean ms of the dominant kernel, clocks)."""
+    """K timed steps, inputs resident: (ms per step, mean ms of the dominant kernel, clocks, keys of the last step)."""
     for _ in range(max(warmup, 3)):
         db.knn2_keys_device(q_dev)
     barrier()
@@ -343,7 +345,7 @@ def time_c4(db, q_dev, steps, warmup, barrier, nat, torch, local_rank):
     e0.record()
     for i in range(steps):
         nat.profile_events(*kern_ev[i])
-        db.knn2_keys_device(q_dev)
+        keys = db.knn2_keys_device(q_dev)
     e1.record()
     barrier()
     nat.profile_events(None, None)
@@ -354,7 +356,18 @@ def time_c4(db, q_dev, steps, warmup, barrier, nat, torch, local_rank):
     if probe:
         clocks["sm_mhz_effective_in_kernel"] = probe["sm_mhz_effective"]
         clocks["effective_note"] = "clock64 / %globaltimer over the first CTA of the last timed k-NN launch"
-    return e0.elapsed_time(e1) / steps, float(np.mean([a.elapsed_time(b) for a, b in kern_ev])), clocks
+    return e0.elapsed_time(e1) / steps, float(np.mean([a.elapsed_time(b) for a, b in kern_ev])), clocks, keys
+
+
+def dump_outputs(out_dir, db, keys, nat):
+    """What a caller of the timed path receives, decoded as `ShardedKeyframeDatabase.knn_tensors` does: imgIdx,
+    trainIdx and distance of the two nearest rows of every query, each [Nq, 2], as float64 (exact for these
+    integers) so that two builds can be compared output for output."""
+    gidx, dist, _ = nat.split_keys(keys.cpu().numpy())
+    img, local = nat.locate_rows(db.starts, gidx)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("img_idx", img), ("train_idx", local), ("distance", dist)):
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float64))
 
 
 def run_b200(args):
@@ -405,7 +418,9 @@ def run_b200(args):
             raise SystemExit("bench: GPU result differs from the oracle")
 
     # ---- timed region: K steps, inputs resident ---------------------------------------------------------
-    ms_per_step, kern_ms, clocks = time_c4(db, q_dev, args.steps, args.warmup, barrier, nat, torch, local_rank)
+    ms_per_step, kern_ms, clocks, last_keys = time_c4(db, q_dev, args.steps, args.warmup, barrier, nat, torch, local_rank)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, db, last_keys, nat)
     t = torch.tensor([ms_per_step, kern_ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -492,7 +507,7 @@ def run_b200(args):
             good = bool(np.array_equal(got[rows], c_oracle.knn2_keys(q2[rows], t2)))
             if not good:
                 raise SystemExit(f"bench: C4 distribution {name}: GPU result differs from the oracle")
-            ms2, k2, _ = time_c4(db2, q2_dev, max(10, args.steps // 4), 3, barrier, nat, torch, local_rank)
+            ms2, k2, _, _ = time_c4(db2, q2_dev, max(10, args.steps // 4), 3, barrier, nat, torch, local_rank)
             others[name] = {"value": total_pairs / (ms2 * 1e-3) / 1e9, "unit": UNIT, "ms_per_step": ms2, "kernel_ms": k2,
                             "verified_rows": int(rows.size)}
             del db2, q2_dev, t2
@@ -554,7 +569,13 @@ def main():
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--quick", action="store_true", help="C4 only: skip the other distributions and the c1/c2/c3/c5 sub-records")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="C4: write what the last timed step computed as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "c4"):
+        ap.error("--dump-outputs applies to the C4 workload of the B200 arm")
     if args.impl == "reference":
         return run_reference(args)
     if args.workload != "c4":

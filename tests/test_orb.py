@@ -200,40 +200,6 @@ def test_frames_described_on_device_match_like_cv2_frames():
         store._ctx.frame_put_orb(0, a[:40], np.zeros((1, 2), np.float32), np.zeros(1, np.float32), np.zeros(1, np.int32))
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/1.png"), reason="build container only: reads the reference's bundled images")
-def test_oracle_describe_on_the_references_own_inputs():
-    """The inputs the survey names for this stage: the bundled pair (C1, 640 x 480 BGR, ORB 200 / 2000 as
-    `/root/reference/slam.py:23` / SURVEY 8(d)) and frames of the C2 warped sequence, regenerated exactly as
-    tests/golden/make_golden_orb.py made them, whose keypoints and descriptors from the UNMODIFIED reference detector
-    are the committed fixture c2_sequence_orb2000.npz.  (These images exist only next to the reference, so this runs
-    where the fixtures were made; the GPU kernels are tied to the oracle on seeded images above.)"""
-    for name in ("1.png", "2.png"):
-        img = cv2.imread(os.path.join("/root/reference", name), flags=cv2.IMREAD_COLOR)
-        for nf in (200, 2000):
-            kps, desc = cv2.ORB.create(nfeatures=nf).detectAndCompute(img, None)
-            assert np.array_equal(oo.describe(img, *kp_arrays(kps)), desc), (name, nf)
-    g = load_golden(os.path.join(GOLDEN, "c2_sequence_orb2000.npz"))
-    rng = np.random.default_rng(752480)
-    base = cv2.resize(cv2.imread("/root/reference/1.png", flags=cv2.IMREAD_GRAYSCALE), (752, 480), interpolation=cv2.INTER_LINEAR)
-    phase = rng.uniform(0, 2 * np.pi, 4)
-    for i in range(3):
-        s = i / 99
-        ang = np.deg2rad(6.0 * np.sin(2 * np.pi * s + phase[0]))
-        tx = 40.0 * np.sin(2 * np.pi * s * 0.7 + phase[1]) + 30.0 * s
-        ty = 25.0 * np.sin(2 * np.pi * s * 0.9 + phase[2])
-        sc = 1.0 + 0.06 * np.sin(2 * np.pi * s * 0.5 + phase[3])
-        c, sn = np.cos(ang) * sc, np.sin(ang) * sc
-        cx, cy = 376.0, 240.0
-        H = np.array([[c, -sn, cx - c * cx + sn * cy + tx], [sn, c, cy - sn * cx - c * cy + ty],
-                      [1e-5 * np.sin(2 * np.pi * s), 8e-6 * np.cos(2 * np.pi * s), 1.0]])
-        frame = cv2.warpPerspective(base, H, (752, 480), flags=cv2.INTER_LINEAR, borderMode=cv2.BORDER_REFLECT101)
-        noisy = np.clip(frame.astype(np.float32) + rng.normal(0.0, 2.0, frame.shape), 0, 255).astype(np.uint8)
-        n = int(g["counts"][i])
-        meta = g["meta"][i, :n]
-        got = oo.describe(noisy, g["points"][i, :n], meta[:, 1], meta[:, 2].astype(np.int32))
-        assert np.array_equal(got, g["descriptors"][i, :n]), i
-
-
 def test_oracle_describe_random_keypoints_all_octaves():
     """Hand-made keypoints at arbitrary sub-pixel positions, angles and octaves (cv2.ORB.compute takes them as given):
     pins the coordinate rounding (pt * (1 / scale), half to even) and the rotation for angles the detector never emits."""
