@@ -891,6 +891,14 @@ static int small_match_run(hm_context* ctx, const uint8_t* q_dev, int64_t nq, co
     return HM_OK;
 }
 
+// hm_small.cu is a POPC kernel: it serves AUTO and POPC calls only, so an explicit tensor-core variant runs the core
+// that was asked for at every size
+static bool small_path(int variant, int64_t nq, int64_t nt)
+{
+    return (variant == HM_VARIANT_AUTO || variant == HM_VARIANT_POPC) && small_match_eligible(nq, nt) &&
+           !(g_prof_start && g_prof_stop);
+}
+
 HM_API int hm_match_host(hm_context* ctx, const uint8_t* query_host, int64_t nq, int64_t q_stride,
                          const uint8_t* train_host, int64_t nt, int64_t t_stride, unsigned flags,
                          const uint16_t* ratio_lut_host, double dist_threshold, int variant, int32_t* out_q_host,
@@ -912,7 +920,7 @@ HM_API int hm_match_host(hm_context* ctx, const uint8_t* query_host, int64_t nq,
     uint8_t *hq = ctx->h_buf, *ht = hq + qb, *hr = ht + tb;
     copy_rows(hq, query_host, nq, q_stride);
     copy_rows(ht, train_host, nt, t_stride);
-    if (small_match_eligible(nq, nt) && !(g_prof_start && g_prof_stop)) {
+    if (small_path(variant, nq, nt)) {
         // one launch, inputs read from the pinned staging buffer, results polled: no copies, no synchronisation
         RatioLut lut;
         int thr;
@@ -1160,7 +1168,7 @@ HM_API int hm_frame_match(hm_context* ctx, int train_slot, int query_slot, unsig
     int32_t* d_pq = d_d + nq;          // 16 + 12 nq bytes: 8-byte aligned when nq is even; padded below otherwise
     if (nq & 1) ++d_pq;
     int32_t* d_pt = d_pq + 2 * nq;
-    if (!want_pts && small_match_eligible(nq, nt) && !(g_prof_start && g_prof_stop)) {
+    if (!want_pts && small_path(variant, nq, nt)) {
         RatioLut lut;
         int thr;
         if ((rc = build_filter_args(flags, ratio_lut_host, dist_threshold, &lut, &thr)) != HM_OK) return rc;
