@@ -53,14 +53,6 @@ def build(force: bool = False, verbose: bool = False) -> str:
         build_hmfast(force)
     except Exception as e:  # pragma: no cover - optional accelerator
         print(f"warning: _hmfast not built ({e}); DMatch construction falls back to Python", file=sys.stderr)
-    trace = os.environ.get("HM_BUILD_TRACE") == "1"
-    if trace:          # separate file: load it with HM_MATCHER_SO=<path> (tools/trace_i8.py does)
-        so = os.path.join(HERE, "libhm_matcher_trace.so")
-        force = True
-    else:
-        so = SO
-    if os.environ.get("HM_BUILD_VARIANT"):
-        force = True
     if not force and not is_stale():
         return SO
     cmd = [
@@ -68,30 +60,14 @@ def build(force: bool = False, verbose: bool = False) -> str:
         "-gencode", "arch=compute_100a,code=sm_100a",
         "--cudart", "static", "-shared", "-Xcompiler", "-fPIC,-fvisibility=hidden",
         "-I", os.path.join(ROOT, "include"), "-I", CSRC,
-        "-o", so,
+        "-o", SO,
     ] + [os.path.join(CSRC, f) for f in SOURCES]
-    if trace:      # pipeline-trace build of the tensor-core kernels
-        cmd.insert(1, "-DHM_TC_TRACE=" + os.environ.get("HM_BUILD_TRACE_STAMPS", "1"))
-        if os.environ.get("HM_BUILD_DEFINE"):          # e.g. HM_BUILD_DEFINE=HM_SPIN_FULL -> libhm_matcher_HM_SPIN_FULL.so
-            cmd.insert(1, "-D" + os.environ["HM_BUILD_DEFINE"])
-            so = os.path.join(HERE, f"libhm_matcher_{os.environ['HM_BUILD_DEFINE'].split('=')[0]}.so")
-            cmd[cmd.index("-o") + 1] = so
-        if os.environ.get("HM_BUILD_EXPERIMENT"):
-            cmd.insert(1, "-DHM_TC_EXPERIMENT=" + os.environ["HM_BUILD_EXPERIMENT"])
-            so = os.path.join(HERE, f"libhm_matcher_exp{os.environ['HM_BUILD_EXPERIMENT']}.so")
-            cmd[cmd.index("-o") + 1] = so
-    variant = os.environ.get("HM_BUILD_VARIANT")
-    if variant and not trace:   # experiment build: HM_BUILD_VARIANT=name HM_BUILD_FLAGS="-DX=1 -DY=2" -> libhm_matcher_<name>.so
-        so = os.path.join(HERE, f"libhm_matcher_{variant}.so")
-        cmd[cmd.index("-o") + 1] = so
-        for f in os.environ.get("HM_BUILD_FLAGS", "").split():
-            cmd.insert(1, f)
     if verbose:
         cmd.insert(1, "-Xptxas")
         cmd.insert(2, "-v")
         print(" ".join(cmd))
     subprocess.check_call(cmd)
-    return so
+    return SO
 
 
 if __name__ == "__main__":

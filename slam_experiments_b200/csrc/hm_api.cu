@@ -80,16 +80,8 @@ inline size_t align_up(size_t v, size_t a = 256) { return (v + a - 1) / a * a; }
 // Static per-shape table (DESIGN.md, "variant selection"): the tensor-core variant pays an
 // operand-expansion pre-pass (two more launches, ~3 us each); kernel-only times (profiles/r01p_probe_shapes.txt):
 // 2000 x 2000 POPC 22 us vs tensor 15 + 6 us, 4096 x 4096 52 us vs 22 + 6 us -- crossover near 8e6 pairs.
-// The tensor-core core AUTO resolves to.  HM_TENSOR_CORE=i8|f4 overrides it for experiments.
-int default_tensor_variant()
-{
-    static int v = 0;
-    if (!v) {
-        const char* e = getenv("HM_TENSOR_CORE");
-        v = (e && !strcmp(e, "i8")) ? HM_VARIANT_I8 : (e && !strcmp(e, "f4")) ? HM_VARIANT_F4 : HM_DEFAULT_TENSOR_VARIANT;
-    }
-    return v;
-}
+// The tensor-core core AUTO resolves to.
+int default_tensor_variant() { return HM_DEFAULT_TENSOR_VARIANT; }
 
 int select_variant(long long nq, long long nt, int batch)
 {
@@ -568,9 +560,8 @@ HM_API int hm_match_fused(const uint8_t* query, int64_t nq, int64_t q_stride, in
     // marks the best train row of every survivor as a candidate; the swapped pass then computes the best query of the
     // CANDIDATE train rows only (gathered inside the kernel from a device-side list).  A match (q, t) is mutual iff q
     // is the best query of t, and only candidates are ever asked -- same result as the full swapped pass, for the
-    // fraction of its work that the ratio test leaves (HM_MUTUAL_FULL=1 forces the full pass, for A/B runs).
-    static const bool full_pass = getenv("HM_MUTUAL_FULL") != nullptr;
-    if (mutual && !full_pass && resolve_variant(variant, nq, nt, batch) == HM_VARIANT_F4) {
+    // fraction of its work that the ratio test leaves.
+    if (mutual && resolve_variant(variant, nq, nt, batch) == HM_VARIANT_F4) {
         SelectArgs sel;
         memset(&sel, 0, sizeof(sel));
         sel.count = reinterpret_cast<int*>(sel_ws);
@@ -736,8 +727,7 @@ static bool same_key(const GraphKey& a, const GraphKey& b)
 template <class F>
 static int run_cached_graph(hm_context* ctx, const GraphKey& key, F&& enqueue)
 {
-    const bool eligible = (double)key.nq * (double)key.nt <= kGraphMaxPairs && !(g_prof_start && g_prof_stop) &&
-                          !getenv("HM_NO_GRAPHS");
+    const bool eligible = (double)key.nq * (double)key.nt <= kGraphMaxPairs && !(g_prof_start && g_prof_stop);
     if (!eligible) return enqueue();
     GraphEntry* e = nullptr;
     for (GraphEntry& g : ctx->graphs)

@@ -215,8 +215,7 @@ size_t small_smem_bytes(long long nq, long long nt) { return (size_t)(nq + nt) *
 
 bool small_match_eligible(long long nq, long long nt)
 {
-    static const bool off = getenv("HM_NO_SMALL_KERNEL") != nullptr;
-    return !off && nq > 0 && nt > 0 && nq <= HM_SMALL_MAX_ROWS && nt <= HM_SMALL_MAX_ROWS && nq * nt <= HM_SMALL_MAX_PAIRS;
+    return nq > 0 && nt > 0 && nq <= HM_SMALL_MAX_ROWS && nt <= HM_SMALL_MAX_ROWS && nq * nt <= HM_SMALL_MAX_PAIRS;
 }
 
 // q / t: device-accessible pointers (device memory or mapped pinned host memory), 32-byte rows, 16-byte aligned;

@@ -47,11 +47,6 @@
 #include "hm_common.cuh"
 #include "hm_tcgen05.cuh"
 
-// train rows per tile of the kind::mxf4 core: 128 (three accumulator units) or 96 (four)
-#ifndef HM_F4_TILE_N
-#define HM_F4_TILE_N 128
-#endif
-
 namespace hm {
 
 namespace {
@@ -63,8 +58,8 @@ constexpr int kBlockM = kRowBlock * kMBlocks;   // 256 queries per CTA
 constexpr int kSlabBytes = kRowBlock * 128;  // 16 KB: 128 rows x 128 bytes of K
 constexpr int kPadRows = HM_PREPARED_TILE_ROWS;
 constexpr int kTmemCols = 512;
-// warp 0 producer, warp 1 MMA issuer, then 4 * kMBlocks * kColSplit epilogue warps: one per 32 query rows
-// and per 128 / kColSplit columns of a tile
+// 4 * kMBlocks * kColSplit epilogue warps (one per 32 query rows and per 128 / kColSplit columns of a tile), then
+// the producer and the MMA issuer
 constexpr uint32_t kSpinLimit = 1u << 26;
 
 static_assert(kPadRows % kBlockM == 0, "prepared padding must cover whole query blocks");
@@ -104,18 +99,12 @@ struct CoreF4 {
     // (4 x 96 = 384 columns) and were tried to give the issuer more slack when an epilogue warp takes the
     // exact-insertion path: bit-exact, but 903 instead of 785 cycles per 128 columns on C4 (per-tile costs of
     // the issuer and of the epilogue warps do not shrink with the tile) -- so 128 rows and three units.
-    static constexpr int kTileN = HM_F4_TILE_N;
-#ifndef HM_F4_STAGES
-#define HM_F4_STAGES 6
-#endif
-    // x 12 / 16 KB in flight.  Six stages (a multiple of the three accumulator units) keep the issuer's unrolled
+    static constexpr int kTileN = 128;
+    // x 16 KB in flight.  Six stages (a multiple of the three accumulator units) keep the issuer's unrolled
     // period at six tiles; 96 KB cover > 4000 cycles of tile time against ~2500 cycles of load latency.
-    static constexpr int kStages = HM_F4_TILE_N == 96 ? 10 : HM_F4_TILE_N == 64 ? 14 : HM_F4_STAGES;
+    static constexpr int kStages = 6;
     // accumulator units of kTileN columns in [0, 480); the scale factors live in the last 32 columns
-#ifndef HM_F4_UNITS
-#define HM_F4_UNITS (HM_F4_TILE_N == 96 ? 5 : HM_F4_TILE_N == 64 ? 7 : 3)
-#endif
-    static constexpr int kUnits = HM_F4_UNITS;
+    static constexpr int kUnits = 3;
     // 16 epilogue warps, two per (query block, lane quarter), 64 columns each: with 8 the scan is latency
     // bound (ncu r01j: issue slots 37 %, ALU 46 %, top stalls wait / long scoreboard) at 1087 cycles per
     // tile while the MMAs need 512
@@ -297,61 +286,7 @@ struct TcParams {
     // few ms, keeps reporting the 1965 MHz application clock while the chip runs the tensor pipe at ~1.65-1.75 GHz.
     long long* clock_probe;
     SelectArgs sel;                  // sel.slot_of != null: ratio test + candidate-column selection on the final keys
-    long long* trace;                // development aid (HM_I8_TRACE): per-tile clock64 stamps of CTA 0, else null
-    int trace_first;                 // first tile recorded (HM_TRACE_FIRST)
 };
-
-// Pipeline trace (development aid): built only with -DHM_TC_TRACE=1 (HM_BUILD_TRACE=1 python -m
-// slam_experiments_b200.build --force), so the shipped kernels carry no trace instructions.
-#ifndef HM_TC_TRACE
-#define HM_TC_TRACE 0
-#endif
-// timing experiments (WRONG RESULTS, development builds only): 1 = epilogue loads and releases the
-// accumulators but does not scan them, 2 = epilogue releases without loading
-#ifndef HM_TC_EXPERIMENT
-#define HM_TC_EXPERIMENT 0
-#endif
-// 1: producer and MMA issuer are the last two warps of the CTA (highest arbitration priority), 0: the first two
-#ifndef HM_ISSUER_LAST
-#define HM_ISSUER_LAST 1
-#endif
-constexpr bool kIssuerLast = HM_ISSUER_LAST != 0;
-// 0: an accumulator unit is committed as soon as its MMAs are issued; 1: both units of a tile are committed at the
-// end of the tile (one pipeline drain per tile instead of two, at the price of signalling block 0 half a tile later)
-#ifndef HM_COMMIT_MODE
-#define HM_COMMIT_MODE 0
-#endif
-constexpr int kTraceTiles = 96;
-constexpr int kTraceSlots = 8;
-// HM_TC_TRACE=2: no per-tile stamps (they perturb the pipeline), only one record per CTA -- globaltimer at entry, after
-// the prologue, at the end of the tile loop, after the final cluster barrier, at exit, and the SM id
-constexpr int kCtaSlots = 24;
-__device__ __forceinline__ void cta_mark(const TcParams& P, int slot)
-{
-#if HM_TC_TRACE
-    if (P.trace) {
-        unsigned long long t;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-        const long long cta = ((long long)blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x;
-        long long* rec = P.trace + kTraceTiles * kTraceSlots + cta * kCtaSlots;
-        rec[slot] = (long long)t;
-        rec[slot + 12] = clock64();          // SM cycles next to wall time: their ratio is the clock actually running
-        if (slot == 0) {
-            unsigned smid;
-            asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-            rec[11] = smid;
-        }
-    }
-#endif
-}
-__device__ __forceinline__ void trace_mark(const TcParams& P, int tile, int slot)
-{
-#if HM_TC_TRACE == 1
-    tile -= P.trace_first;
-    if (P.trace && blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == 0 && tile >= 0 && tile < kTraceTiles)
-        P.trace[tile * kTraceSlots + slot] = clock64();
-#endif
-}
 
 // Running top-2 of one query row at GROUP granularity.  A group is 8 consecutive train columns.  The scan keeps the
 // two groups with the largest maxima (earliest group on ties) and a copy of their 8 dots each, packed two per
@@ -373,9 +308,6 @@ struct Top2 {
     // one compare against f skips everything else.  v2 only grows, so after an insertion
     // max(v2_new, shared) = max(v2_new, f_old) and `shared` itself need not be kept.
     Acc f;
-#if HM_TC_TRACE
-    unsigned slow;                   // trace builds: warp-level entries into the insertion path
-#endif
 };
 
 __device__ __forceinline__ void bounded_wait(uint64_t* bar, uint32_t parity, int* error_flag)
@@ -407,16 +339,12 @@ __device__ __forceinline__ void tmem_ld_fence4(uint32_t (&a)[32], uint32_t (&b)[
 {
     asm volatile("tcgen05.wait::ld.sync.aligned;\n" : HM_R32(a), HM_R32(b), HM_R32(c), HM_R32(d) : : "memory");
 }
-__device__ __forceinline__ void tmem_ld_fence48(uint32_t (&a)[32], uint32_t (&b)[16])
-{
-    asm volatile("tcgen05.wait::ld.sync.aligned;\n" : HM_R32(a), HM_R8(b, 0), HM_R8(b, 8) : : "memory");
-}
 __device__ __forceinline__ void tmem_ld_fence64(uint32_t (&a)[64])
 {
     asm volatile("tcgen05.wait::ld.sync.aligned;\n" : HM_R8(a, 0), HM_R8(a, 8), HM_R8(a, 16), HM_R8(a, 24), HM_R8(a, 32), HM_R8(a, 40), HM_R8(a, 48), HM_R8(a, 56) : : "memory");
 }
 
-// 32 (16) consecutive train columns of one query row.  Fast path: 3-input-max trees give the maximum of each group
+// 32 (64) consecutive train columns of one query row.  Fast path: 3-input-max trees give the maximum of each group
 // of 8 columns and of the whole chunk; one compare + branch per chunk against the threshold decides whether anything
 // can change the top-2.  Only then are the group maxima revisited; a group above the threshold is inserted into the
 // top-2 of groups together with a packed copy of its dots.  Strict '>' in ascending column order keeps the earliest
@@ -428,7 +356,7 @@ template <class C, int kMode, int kGroups = 4>
 __device__ __forceinline__ void scan_chunk(const uint32_t* r, unsigned colbase, Top2<typename C::Acc>& s)
 {
     using Acc = typename C::Acc;
-    static_assert(kGroups == 2 || kGroups == 4 || kGroups == 8, "8-column groups per compare");
+    static_assert(kGroups == 4 || kGroups == 8, "8-column groups per compare");
     Acc gm[kGroups];
 #pragma unroll
     for (int g = 0; g < kGroups; ++g) {
@@ -439,13 +367,9 @@ __device__ __forceinline__ void scan_chunk(const uint32_t* r, unsigned colbase, 
     }
     Acc m;
     if constexpr (kGroups == 8) m = C::max3(C::max3(gm[0], gm[1], gm[2]), C::max3(gm[3], gm[4], gm[5]), C::max2(gm[6], gm[7]));
-    else if constexpr (kGroups == 4) m = C::max3(gm[0], gm[1], C::max2(gm[2], gm[3]));
-    else m = C::max2(gm[0], gm[1]);
+    else m = C::max3(gm[0], gm[1], C::max2(gm[2], gm[3]));
     constexpr bool kFloor = kMode == 1, kTop1 = kMode == 2;
     if (m > (kFloor ? s.f : kTop1 ? s.v1 : s.v2)) {
-#if HM_TC_TRACE
-        s.slow += 1;
-#endif
 #pragma unroll
         for (int g = 0; g < kGroups; ++g) {
             const Acc x = gm[g];
@@ -482,35 +406,9 @@ __device__ __forceinline__ void mask_tail(uint32_t* r, unsigned colbase, unsigne
     }
 }
 
-// 1: the epilogue thread that releases an accumulator unit is picked with elect.sync, 0: lane 0
-#ifndef HM_ARRIVE_ELECT
-#define HM_ARRIVE_ELECT 1
-#endif
-// 1: the kind::mxf4 epilogue scans its 64 columns with one compare + branch, 0: as two 32-column chunks
-#ifndef HM_SCAN_FLAT64
-#define HM_SCAN_FLAT64 1
-#endif
-// tiles of a CTA during which the shared row thresholds are refreshed every tile (every 16th afterwards)
-#ifndef HM_FLOOR_DENSE_TILES
-#define HM_FLOOR_DENSE_TILES 32
-#endif
-#ifndef HM_FLOOR_LATE_MASK
-#define HM_FLOOR_LATE_MASK 15
-#endif
-
-// EXPERIMENT, OFF: 1 (kind::mxf4 only) keeps the A operand (the CTA's 256 query rows) in tensor memory, 32 columns per
-// 128-row block, written once by the epilogue warps; the MMAs then read only B from shared memory, which halves the
-// tensor core's shared-memory operand traffic (A + B from shared memory is 128 B/clk/SM, the whole shared-memory
-// bandwidth).  It is 2.6 % faster on C4 (690 -> 672 cycles per tile) and passes the parity suite most of the time --
-// but NOT always: tools/repro_c4.py finds 1-3 wrong rows (a true neighbour missed in one late tile) in 4-9 of 30
-// full-size C4 launches, never with A in shared memory.  Something about tcgen05.mma reading A from tensor memory
-// while tcgen05.ld drains other columns is not covered by the fences used here; until that is understood the
-// operand stays in shared memory.
-#ifndef HM_F4_A_TMEM
-#define HM_F4_A_TMEM 0
-#endif
-constexpr int kATmemCol = 384;                       // [384, 448): after three 128-column accumulator units
-constexpr int kATmemColsPerBlock = 32;               // 256 e2m1 = 128 bytes per row
+// the shared row thresholds are refreshed on each of a CTA's first kFloorDenseTiles tiles, then on every 16th
+constexpr int kFloorDenseTiles = 32;
+constexpr int kFloorLateMask = 15;
 
 // half `h` (0 / 1) of the MMAs of one (tile, query block) item: kSlabs * 2 instructions
 template <class C>
@@ -524,14 +422,9 @@ __device__ __forceinline__ void issue_half(int h, uint32_t a_block, uint32_t b_s
         const int slab = j >> 2, k = j & 3;
         // a_block / b_stage are descriptor start-address fields (shared-memory address >> 4)
         const uint64_t db = ptx::kmajor_sw128_desc_from_lo(b_stage + ((slab * kSlabBytes + k * 32) >> 4));
-        if constexpr (C::kScales && HM_F4_A_TMEM) {
-            // a_block is the TMEM address of the block's first A column; K = 64 elements = 8 columns per instruction
-            ptx::mma_mxf4_ts(tmem_d, a_block + 8 * j, db, idesc, tmem_sf, tmem_sf + kScaleCols / 2, j != 0);
-        } else {
-            const uint64_t da = ptx::kmajor_sw128_desc_from_lo(a_block + ((slab * kSlabBytes + k * 32) >> 4));
-            if constexpr (C::kScales) ptx::mma_mxf4_ss(tmem_d, da, db, idesc, tmem_sf, tmem_sf + kScaleCols / 2, j != 0);
-            else                      ptx::mma_i8_ss(tmem_d, da, db, idesc, j != 0);
-        }
+        const uint64_t da = ptx::kmajor_sw128_desc_from_lo(a_block + ((slab * kSlabBytes + k * 32) >> 4));
+        if constexpr (C::kScales) ptx::mma_mxf4_ss(tmem_d, da, db, idesc, tmem_sf, tmem_sf + kScaleCols / 2, j != 0);
+        else                      ptx::mma_i8_ss(tmem_d, da, db, idesc, j != 0);
     }
 }
 
@@ -566,7 +459,6 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
     // broadcast from lane 0: lets ptxas treat the warp index (and the role branches on it) as warp-uniform
     const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0);
     const int lane = threadIdx.x & 31;
-    if (threadIdx.x == 0) cta_mark(P, 0);
     if (threadIdx.x == 0 && (blockIdx.x | blockIdx.y | blockIdx.z) == 0 && P.clock_probe) {
         unsigned long long t;
         asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
@@ -595,10 +487,8 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
     // (/opt/skills/guides/B300_MICROARCH.md, "Multi-warp arbiter"), so the two latency-critical single warps -- the
     // MMA issuer above all -- are the LAST two warps of the CTA: the issuer never queues behind the four epilogue
     // warps that share its sub-partition.  Epilogue warps come first; warp % 4 is still their TMEM lane quarter.
-    constexpr int kProducerWarp = kIssuerLast ? epilogue_warps<C>() : 0;
-    constexpr int kIssuerWarp = kIssuerLast ? epilogue_warps<C>() + 1 : 1;
-    constexpr int kFirstEpiWarp = kIssuerLast ? 0 : 2;
-    static_assert(kIssuerLast || !C::kRegisterHandover, "the control warps must form the last warpgroup");
+    constexpr int kProducerWarp = epilogue_warps<C>();
+    constexpr int kIssuerWarp = epilogue_warps<C>() + 1;
     static_assert(!C::kRegisterHandover || (epilogue_warps<C>() == 16 && threads<C>() == 640),
                   "the register budget (4 x 32 + 16 x 112 = 20 x 96) assumes 20 warps launched at 96 registers");
     if (warp == kProducerWarp && lane == 0) {
@@ -626,7 +516,7 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
 
     if constexpr (C::kScales) {
         // every block scale is 1.0 (ue8m0 0x7F): fill the scale-factor columns once, all 128 lanes
-        if (warp >= kFirstEpiWarp && warp < kFirstEpiWarp + 4) {
+        if ((unsigned)warp < 4) {          // the first four epilogue warps, one per lane quarter
             uint32_t ones[32];
 #pragma unroll
             for (int i = 0; i < 32; ++i) ones[i] = 0x7F7F7F7Fu;
@@ -635,45 +525,7 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
             ptx::tmem_st_32x32(taddr, ones);
             ptx::tmem_st_wait();
         }
-        if (HM_F4_A_TMEM) {
-            // A operand into tensor memory: thread = query row (TMEM lane), 32 words = the row's 256 e2m1 values in
-            // logical order; one tcgen05.st per (128-row block, lane quarter), by the warps of the lower column half
-            static_assert(!HM_F4_A_TMEM || C::kUnits * C::kTileN <= kATmemCol, "accumulator units overlap the A operand");
-            static_assert(!HM_F4_A_TMEM || kATmemCol + kMBlocks * kATmemColsPerBlock <= kScaleCol, "A operand overlaps the scale factors");
-            if (warp >= kFirstEpiWarp && warp < kFirstEpiWarp + 4 * kMBlocks) {
-                const int wq = warp & 3, wblk = ((warp - kFirstEpiWarp) >> 2) & 1;
-                const int r = wq * 32 + lane;
-                const long long qrow = (long long)qb * kBlockM + wblk * kRowBlock + r;
-                uint32_t words[32];
-#pragma unroll
-                for (int i = 0; i < 32; ++i) words[i] = 0u;
-                if (qrow < rows_present()) {
-                    if (P.qbits) {
-                        const int* qidx = P.q_index ? P.q_index + (long long)b * P.q_index_batch_stride : nullptr;
-                        const long long srow = qidx ? (long long)__ldg(qidx + qrow) : qrow;
-                        const uint4* src = reinterpret_cast<const uint4*>(P.qbits + (long long)b * P.q_bits_batch_stride + srow * P.q_bits_stride);
-                        const uint4 lo = src[0], hi = src[1];
-                        const unsigned bits[8] = {lo.x, lo.y, lo.z, lo.w, hi.x, hi.y, hi.z, hi.w};
-#pragma unroll
-                        for (int c = 0; c < 8; ++c) {
-                            const uint4 v = expand_bits_e2m1(bits[c]);
-                            words[4 * c] = v.x; words[4 * c + 1] = v.y; words[4 * c + 2] = v.z; words[4 * c + 3] = v.w;
-                        }
-                    } else if (has_a) {
-                        // prepared image: 8-row atoms of 1024 bytes, logical 16-byte chunk c of row r at position c ^ (r & 7)
-                        const uint8_t* img = P.qprep + ((long long)b * P.q_padded + (long long)qb * kBlockM + wblk * kRowBlock) * C::kRowBytes;
-                        const uint4* row = reinterpret_cast<const uint4*>(img + (r >> 3) * 1024 + (r & 7) * 128);
-#pragma unroll
-                        for (int c = 0; c < 8; ++c) {
-                            const uint4 v = row[c ^ (r & 7)];
-                            words[4 * c] = v.x; words[4 * c + 1] = v.y; words[4 * c + 2] = v.z; words[4 * c + 3] = v.w;
-                        }
-                    }
-                }
-                ptx::tmem_st_32x32(tmem_base + ((uint32_t)(wq * 32) << 16) + kATmemCol + wblk * kATmemColsPerBlock, words);
-                ptx::tmem_st_wait();
-            }
-        } else if (P.qbits) {
+        if (P.qbits) {
             // A operand from packed bits: the same swizzled image hm_prepare_f4_kernel writes, straight into shared
             // memory (chunk position -> row and logical chunk as there); rows past nq are +0.0 like the padding
             const uint8_t* qsrc = P.qbits + (long long)b * P.q_bits_batch_stride;
@@ -699,7 +551,6 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
         ptx::tc_fence_after();
     }
 
-    if (threadIdx.x == 0) cta_mark(P, 1);
     ulonglong2 my_keys = make_ulonglong2(kNoMatch, kNoMatch);   // epilogue threads: top-2 keys of their row (and column half)
     long long my_row = -1;                                      // >= 0: this thread writes the row's keys
     int my_row_in_cta = 0;
@@ -709,20 +560,17 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
     auto run_producer = [&]() {
         // ===== producer: bulk async copies global -> shared =====
         if (lane == 0) {
-            if (has_a && !P.qbits && !(C::kScales && HM_F4_A_TMEM)) {
+            if (has_a && !P.qbits) {
                 const uint8_t* qsrc = P.qprep + ((long long)b * P.q_padded + (long long)qb * kBlockM) * C::kRowBytes;
                 ptx::mbar_arrive_expect_tx(a_full_bar, kABytes);
                 ptx::bulk_g2s(smem_a, qsrc, kABytes, a_full_bar);       // two consecutive row blocks
             }
             const uint8_t* tsrc = P.tprep + (long long)b * P.t_padded * C::kRowBytes;
             const uint32_t piece = kBStageBytes / cs;     // this CTA fetches 1/cs of every tile and multicasts it
-            for (int i = 0; i < (HM_TC_EXPERIMENT >= 5 ? 0 : my_tiles); ++i) {
+            for (int i = 0; i < my_tiles; ++i) {
                 const int stage = i % kStages;
                 const uint32_t use = i / kStages;
-#if HM_TC_EXPERIMENT < 4
                 bounded_wait(&empty_bar[stage], (use & 1) ^ 1, P.error_flag);
-#endif
-                trace_mark(P, i, 0);                      // producer: stage free, copy issued
                 ptx::mbar_arrive_expect_tx(&full_bar[stage], kBStageBytes);
                 uint8_t* dst = smem_b + stage * kBStageBytes + crank * piece;
                 const uint8_t* src = tsrc + (long long)(tile_begin + i) * kBStageBytes + crank * piece;
@@ -751,12 +599,11 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
         // and blocking waits instead of the probes cost 70 cycles per tile.)
         const bool leader = ptx::elect_one();
         const uint32_t idesc = C::kScales ? ptx::make_mxf4_idesc(kRowBlock, kTileN) : ptx::make_i8_idesc(kRowBlock, kTileN);
-        constexpr bool kATmem = C::kScales && HM_F4_A_TMEM;
-        const uint32_t a_addr = kATmem ? tmem_base + kATmemCol : ptx::smem_u32(smem_a) >> 4;       // TMEM address / descriptor start-address field
-        constexpr uint32_t kABlockStep = kATmem ? (uint32_t)kATmemColsPerBlock : (uint32_t)(kRowBlockBytes >> 4);
+        const uint32_t a_addr = ptx::smem_u32(smem_a) >> 4;       // descriptor start-address fields
+        constexpr uint32_t kABlockStep = kRowBlockBytes >> 4;
         const uint32_t b_addr = ptx::smem_u32(smem_b) >> 4;
         const uint32_t tmem_sf = tmem_base + kScaleCol;
-        if (has_a && !P.qbits && !(C::kScales && HM_F4_A_TMEM)) bounded_wait(a_full_bar, 0, P.error_flag);
+        if (has_a && !P.qbits) bounded_wait(a_full_bar, 0, P.error_flag);
         // The loop is unrolled over one period of the stage ring and of the unit rotation (kPeriod tiles), so that the
         // stage, the accumulator units, every barrier address, every descriptor offset and the unit parities are
         // compile-time constants: what is left per tile is the eight (sixteen) MMAs, three commits, the probes / waits
@@ -777,54 +624,31 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
                     const int unit_a = (2 * j) % kUnits, unit_b = (2 * j + 1) % kUnits;
                     const uint32_t par_a = (((2 * j) / kUnits) & 1) ^ 1, par_b = (((2 * j + 1) / kUnits) & 1) ^ 1;
                     const uint32_t b_stage = b_addr + stage * (kBStageBytes >> 4);
-                    if (leader) trace_mark(P, base + j, 7);           // loop top
                     if (!ready0) {
-#if HM_TC_EXPERIMENT < 4
                         bounded_wait(&full_bar[stage], full_par, P.error_flag);
-#endif
-#if HM_TC_EXPERIMENT < 3
                         bounded_wait(&tmem_empty_bar[unit_a], par_a, P.error_flag);
-#endif
                     }
-                    if (leader) trace_mark(P, base + j, 1);           // operands landed, first unit free
                     ptx::tc_fence_after();
                     // ---- query block 0 ----
                     if (leader) issue_half<C>(0, a_addr, b_stage, tmem_base + unit_a * kTileN, idesc, tmem_sf);
-#if HM_TC_EXPERIMENT >= 3
-                    const bool ready1 = true;
-#else
                     const bool ready1 = __all_sync(0xffffffffu, ptx::mbar_test_wait(&tmem_empty_bar[unit_b], par_b));
-#endif
                     if (leader) {
                         issue_half<C>(1, a_addr, b_stage, tmem_base + unit_a * kTileN, idesc, tmem_sf);
-#if HM_TC_EXPERIMENT != 6 && HM_COMMIT_MODE == 0
                         ptx::tc_commit(&tmem_full_bar[unit_a]);    // query block 0's accumulator is ready
-#endif
                     }
                     // ---- query block 1 ----
                     if (!ready1) bounded_wait(&tmem_empty_bar[unit_b], par_b, P.error_flag);
-                    if (leader) trace_mark(P, base + j, 6);           // second unit free
                     ptx::tc_fence_after();
                     if (leader) issue_half<C>(0, a_addr + kABlockStep, b_stage, tmem_base + unit_b * kTileN, idesc, tmem_sf);
                     ready0 = false;
                     if (base + j + 1 < my_tiles) {
                         const int n = j + 1;                       // n == kPeriod wraps to stage 0 / unit 0 of the next period
-#if HM_TC_EXPERIMENT >= 4
-                        ready0 = true;
-#else
                         ready0 = __all_sync(0xffffffffu,
                                             ptx::mbar_test_wait(&full_bar[n % kStages], sphase ^ ((n / kStages) & 1))
-#if HM_TC_EXPERIMENT < 3
-                                            && ptx::mbar_test_wait(&tmem_empty_bar[(2 * n) % kUnits], (((2 * n) / kUnits) & 1) ^ 1)
-#endif
-                                            );
-#endif
+                                            && ptx::mbar_test_wait(&tmem_empty_bar[(2 * n) % kUnits], (((2 * n) / kUnits) & 1) ^ 1));
                     }
                     if (leader) {
                         issue_half<C>(1, a_addr + kABlockStep, b_stage, tmem_base + unit_b * kTileN, idesc, tmem_sf);
-#if HM_TC_EXPERIMENT == 6 || HM_COMMIT_MODE == 1
-                        ptx::tc_commit(&tmem_full_bar[unit_a]);
-#endif
                         ptx::tc_commit(&tmem_full_bar[unit_b]);
                         // smem stage reusable (by every producer of the cluster) once these MMAs retire
                         if (cs > 1) ptx::tc_commit_multicast(&empty_bar[stage], cmask);
@@ -840,8 +664,8 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
         // ===== epilogue: TMEM -> registers, running top-2 per query row =====
         constexpr int kCols = kTileN / C::kColSplit;      // train columns of a tile this warp scans
         const int quarter = warp & 3;                     // TMEM lanes [32*quarter, +32) belong to this warp
-        const int mblk = ((warp - kFirstEpiWarp) >> 2) & 1;   // which 128-row query block of the CTA
-        const int half = (warp - kFirstEpiWarp) >> 3;         // which column range of every tile (0 when kColSplit == 1)
+        const int mblk = (warp >> 2) & 1;                 // which 128-row query block of the CTA
+        const int half = warp >> 3;                       // which column range of every tile (0 when kColSplit == 1)
         const int row_in_cta = mblk * kRowBlock + quarter * 32 + lane;
         const long long row = (long long)qb * kBlockM + row_in_cta;
         Top2<Acc> s;
@@ -850,9 +674,6 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
 #pragma unroll
         for (int e = 0; e < 4; ++e) s.sa[e] = s.sb[e] = 0;
         s.f = C::floor_from(0);                           // below every possible dot
-#if HM_TC_TRACE
-        s.slow = 0;
-#endif
         unsigned floor_code = 0;                          // largest threshold code read or published so far
         const long long first_row = (long long)tile_begin * kTileN;
         const unsigned limit = (unsigned)min((long long)my_tiles * kTileN, P.nt - first_row);
@@ -872,7 +693,7 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
         unsigned floor_pending = 0;
         auto refresh_floor = [&](int i) {
             if constexpr (kFloor) {
-                if (i < HM_FLOOR_DENSE_TILES || (i & HM_FLOOR_LATE_MASK) == 0) {
+                if (i < kFloorDenseTiles || (i & kFloorLateMask) == 0) {
                     floor_code = max(floor_code, floor_pending);
                     s.f = C::max2(s.f, C::floor_from(floor_code));
                     if (row < P.nq) {              // (the threshold kernels never run with a device-side row count)
@@ -886,11 +707,6 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
         };
         auto process_tile = [&](int i) {
             bounded_wait_addr(unit_full_addr + unit * 8, unit_use & 1, P.error_flag);
-#if HM_TC_TRACE == 2
-            if (warp == kFirstEpiWarp && lane == 0 && (i == 8 || i == 32 || i == 64 || i == 192)) cta_mark(P, i == 8 ? 5 : i == 32 ? 6 : i == 64 ? 7 : 8);
-#endif
-            if (warp == kFirstEpiWarp && lane == 0) trace_mark(P, i, 3);   // epilogue: accumulator complete
-            if (warp == kFirstEpiWarp + 7 && lane == 0) trace_mark(P, i, 5);
             ptx::tc_fence_after();
             const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + unit * kTileN + half * kCols;
             const unsigned colbase = (unsigned)i * kTileN + half * kCols;
@@ -906,7 +722,7 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
                 // the accumulator unit is in registers: release it before the scan
                 ptx::tc_fence_before();
                 __syncwarp();
-                if (HM_ARRIVE_ELECT ? ptx::elect_one() : lane == 0) ptx::mbar_arrive_addr(unit_empty_addr + unit * 8);
+                if (ptx::elect_one()) ptx::mbar_arrive_addr(unit_empty_addr + unit * 8);
                 if (colbase + kCols > limit) {            // last tile of the train set only
                     mask_tail<C, 32>(r0, colbase, limit);
                     mask_tail<C, 32>(r1, colbase + 32, limit);
@@ -918,74 +734,26 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
                 scan_chunk<C, kMode>(r2, colbase + 64, s);
                 scan_chunk<C, kMode>(r3, colbase + 96, s);
             } else {
-                if constexpr (kCols == 64) {
-                    uint32_t r[64];
-#if HM_TC_EXPERIMENT < 2
-                    ptx::tmem_ld_32x64(taddr, r);
-                    refresh_floor(i);
-                    tmem_ld_fence64(r);
-#endif
-                    ptx::tc_fence_before();
-                    __syncwarp();
-                    if (HM_ARRIVE_ELECT ? ptx::elect_one() : lane == 0) ptx::mbar_arrive_addr(unit_empty_addr + unit * 8);
-#if HM_TC_EXPERIMENT != 0
-                    unit += 2;
-                    if (unit >= kUnits) { unit -= kUnits; ++unit_use; }
-                    return;
-#endif
-                    // (tried and slower, C4 cycles per tile against 785: one flat 64-column tree with a single branch 867;
-                    // warp-uniform votes around the insertion path 871; software pipelining over half items -- two
-                    // 32-register buffers, the next item's first half loaded while this item's second half is
-                    // scanned -- 882)
-                    mask_tail<C, 64>(r, colbase, limit);
-#if HM_SCAN_FLAT64
-                    scan_chunk<C, kMode, 8>(r, colbase, s);          // one compare + branch per 64 columns
-#else
-                    scan_chunk<C, kMode>(r, colbase, s);
-                    scan_chunk<C, kMode>(r + 32, colbase + 32, s);
-#endif
-                } else if constexpr (kCols == 32) {
-                    uint32_t r[32];
-                    ptx::tmem_ld_32x32(taddr, r);
-                    refresh_floor(i);
-                    asm volatile("tcgen05.wait::ld.sync.aligned;\n" : HM_R32(r) : : "memory");
-                    ptx::tc_fence_before();
-                    __syncwarp();
-                    if (HM_ARRIVE_ELECT ? ptx::elect_one() : lane == 0) ptx::mbar_arrive_addr(unit_empty_addr + unit * 8);
-                    mask_tail<C, 32>(r, colbase, limit);
-                    scan_chunk<C, kMode>(r, colbase, s);
-                } else {
-                    static_assert(kCols == 64 || kCols == 48, "column split");
-                    uint32_t r0[32], r1[16];
-                    ptx::tmem_ld_32x32(taddr, r0);
-                    ptx::tmem_ld_32x16(taddr + 32, r1);
-                    refresh_floor(i);
-                    tmem_ld_fence48(r0, r1);
-                    ptx::tc_fence_before();
-                    __syncwarp();
-                    if (HM_ARRIVE_ELECT ? ptx::elect_one() : lane == 0) ptx::mbar_arrive_addr(unit_empty_addr + unit * 8);
-                    mask_tail<C, 32>(r0, colbase, limit);
-                    mask_tail<C, 16>(r1, colbase + 32, limit);
-                    scan_chunk<C, kMode>(r0, colbase, s);
-                    scan_chunk<C, kMode, 2>(r1, colbase + 32, s);
-                }
+                static_assert(kCols == 64, "column split");
+                uint32_t r[64];
+                ptx::tmem_ld_32x64(taddr, r);
+                refresh_floor(i);
+                tmem_ld_fence64(r);
+                ptx::tc_fence_before();
+                __syncwarp();
+                if (ptx::elect_one()) ptx::mbar_arrive_addr(unit_empty_addr + unit * 8);
+                // (tried and slower, C4 cycles per tile against 785: warp-uniform votes around the insertion path 871;
+                // software pipelining over half items -- two 32-register buffers, the next item's first half loaded
+                // while this item's second half is scanned -- 882.  The flat 64-column tree below measured 867 then;
+                // with the group-level scan it measured a wash and was adopted, DESIGN.md §3.3 items 10-11.)
+                mask_tail<C, 64>(r, colbase, limit);
+                scan_chunk<C, kMode, 8>(r, colbase, s);          // one compare + branch per 64 columns
             }
             unit += 2;
             if (unit >= kUnits) { unit -= kUnits; ++unit_use; }
-            if (warp == kFirstEpiWarp && lane == 0) trace_mark(P, i, 4);   // epilogue: buffer released
         };
 #pragma unroll 1
         for (int i = 0; i < my_tiles; ++i) process_tile(i);
-        if (warp == kFirstEpiWarp && lane == 0) cta_mark(P, 2);
-#if HM_TC_TRACE
-        if (P.trace) {   // slot 9: warp-chunks of this CTA in which at least one lane took the exact-insertion path; slot 10: lane events
-            const long long cta = ((long long)blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x;
-            long long* rec = P.trace + kTraceTiles * kTraceSlots + cta * kCtaSlots;
-            const unsigned any = __reduce_max_sync(0xffffffffu, s.slow);   // not exact (max over lanes) but a lower bound of warp events
-            const unsigned sum = __reduce_add_sync(0xffffffffu, s.slow);
-            if (lane == 0) { atomicAdd((unsigned long long*)&rec[9], (unsigned long long)any); atomicAdd((unsigned long long*)&rec[10], (unsigned long long)sum); }
-        }
-#endif
         const unsigned long long gbase = P.train_base + (unsigned long long)first_row;
         // exact top-2 from the saved dots of the two best groups (u64 min over (distance, trainIdx) keys = cv2's order)
         auto fold_group = [&](Acc v, unsigned i0, const uint32_t (&p)[4]) {
@@ -1010,7 +778,6 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
         ptx::tc_fence_before();
         if (cs > 1) ptx::cluster_sync();   // no CTA leaves while peers may still signal its barriers
         else __syncthreads();
-        if (kWorker && threadIdx.x == 0) cta_mark(P, 3);
         if (warp == kIssuerWarp) {
             ptx::tc_fence_after();
             ptx::tmem_dealloc(tmem_base, kTmemCols);
@@ -1043,7 +810,6 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
                 }
             }
         }
-        if (kWorker && threadIdx.x == 0) cta_mark(P, 4);
         if (kWorker && threadIdx.x == 0 && (blockIdx.x | blockIdx.y | blockIdx.z) == 0 && P.clock_probe) {
             unsigned long long t;
             asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
@@ -1095,30 +861,8 @@ struct TcPlan {
     long long qblocks;               // grid.x, rounded up to a multiple of `cluster`
 };
 
-// split launches whose CTAs have at most this many tiles use the shared-row-threshold kernels (HM_FLOOR_MAX_TILES
-// overrides for experiments)
-int floor_max_tiles()
-{
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("HM_FLOOR_MAX_TILES");
-        v = e ? atoi(e) : 0x7fffffff;
-    }
-    return v;
-}
-
-// unsplit launches use the floor kernels (thresholds shared by the two column-half warps of a row) from this
-// many tiles per CTA on (HM_FLOOR_MIN_TILES_UNSPLIT overrides; 0x7fffffff = never)
-int floor_min_tiles_unsplit()
-{
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("HM_FLOOR_MIN_TILES_UNSPLIT");
-        v = e ? atoi(e) : 0x7fffffff;
-    }
-    return v;
-}
-
+// test hook: HM_I8_CLUSTER=1|2|4 forces the cluster size of every tensor-core launch of the process, so that tests can
+// run cluster shapes the planner would not choose for their problem size
 int cluster_override()
 {
     static int v = -1;
@@ -1196,29 +940,6 @@ int resident_ctas(int cs, int sm_count)
     return v;
 }
 
-// fixed per-CTA cost in steady-state tile times (HM_PROLOGUE_TILES overrides, for planner sweeps)
-template <class C>
-int prologue_tiles()
-{
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("HM_PROLOGUE_TILES");
-        v = e ? atoi(e) : C::kPrologueTiles;
-    }
-    return v;
-}
-
-// clusters of 2 pay from this many tiles per CTA on (HM_CLUSTER_MIN_TILES overrides, for sweeps)
-int cluster_min_tiles()
-{
-    static int v = -1;
-    if (v < 0) {
-        const char* e = getenv("HM_CLUSTER_MIN_TILES");
-        v = e ? atoi(e) : 1024;
-    }
-    return v;
-}
-
 template <class C>
 TcPlan plan_tc_cluster(long long nq, long long nt, int batch, int sm_count, int cluster)
 {
@@ -1237,7 +958,7 @@ TcPlan plan_tc_cluster(long long nq, long long nt, int batch, int sm_count, int 
         const long long tps = ceil_div(pl.ntiles, s);
         const long long real_s = ceil_div(pl.ntiles, tps);
         const long long waves = ceil_div(items * real_s, sm_count);
-        const long long cost = waves * (tps + prologue_tiles<C>());
+        const long long cost = waves * (tps + C::kPrologueTiles);
         if (best_cost < 0 || cost < best_cost) {
             best_cost = cost;
             best = s;
@@ -1256,10 +977,12 @@ TcPlan plan_tc(long long nq, long long nt, int batch, int sm_count)
     // Pairs of query blocks share every train tile through multicast: half the L2 reads, 1.7 % on C4 (690 vs 702 cycles
     // per tile at 1730 tiles per CTA; clusters of 4 lose SMs to GPC packing: 747).  CTAs that see few tiles gain nothing
     // from it and schedule better alone: C5 (79 tiles per CTA) +2 %, C2 (16) +2.5 %, 16k x 16k +2.5 %, and a wash for
-    // the 2000-query shards of the multi-GPU runs (445-889 tiles: within 0.7 %).
+    // the 2000-query shards of the multi-GPU runs (445-889 tiles: within 0.7 %).  Clusters of 2 therefore pay from this
+    // many tiles per CTA on:
+    constexpr int kClusterMinTiles = 1024;
     if (ceil_div(nq, kBlockM) >= 2) {
         const TcPlan pl = plan_tc_cluster<C>(nq, nt, batch, sm_count, 2);
-        if (pl.tiles_per_split >= cluster_min_tiles()) return pl;
+        if (pl.tiles_per_split >= kClusterMinTiles) return pl;
     }
     return plan_tc_cluster<C>(nq, nt, batch, sm_count, 1);
 }
@@ -1335,13 +1058,6 @@ int launch_prepared(const void* qprep, long long nq, const void* tprep, long lon
     P.error_flag = static_cast<int*>(ws);
     P.clock_probe = reinterpret_cast<long long*>(static_cast<uint8_t*>(ws) + HM_WS_CLOCK_PROBE_OFFSET);   // inside the 256-byte header
     P.q_blocks_valid = P.q_padded / kBlockM;
-    const char* trace_path = getenv("HM_I8_TRACE");
-    if (trace_path) {
-        if (const char* tf = getenv("HM_TRACE_FIRST")) P.trace_first = atoi(tf);
-        const size_t trace_words = (size_t)kTraceTiles * kTraceSlots + (size_t)pl.qblocks * pl.splits * batch * kCtaSlots;
-        HM_CUDA_CHECK(cudaMalloc(&P.trace, sizeof(long long) * trace_words));
-        HM_CUDA_CHECK(cudaMemset(P.trace, 0, sizeof(long long) * trace_words));
-    }
     const long long rows = nq * batch;
     unsigned* counters = reinterpret_cast<unsigned*>(static_cast<uint8_t*>(ws) + 256);
     unsigned long long* partials = reinterpret_cast<unsigned long long*>(static_cast<uint8_t*>(ws) + 256 + cbytes);
@@ -1361,10 +1077,10 @@ int launch_prepared(const void* qprep, long long nq, const void* tprep, long lon
         P.out = partials;                  // even with one split: the exchange runs in the last-CTA path
         P.out_split_stride = rows * 2;
     }
-    // shared row thresholds: the CTAs (and, with kColSplit == 2, the two column-half warps) of a query row
+    // shared row thresholds: between the CTAs of a query row in split launches (and, with kColSplit == 2, between the
+    // two column-half warps of the row in each CTA)
     bool zero_block = false;
-    const bool floor_eligible = !top1 && !P.nq_dyn && pl.tiles_per_split <= floor_max_tiles() &&
-                                (pl.splits > 1 || (C::kColSplit > 1 && pl.ntiles >= floor_min_tiles_unsplit()));
+    const bool floor_eligible = !top1 && !P.nq_dyn && pl.splits > 1;
     if (floor_eligible) {
         P.row_floor = reinterpret_cast<unsigned*>(reinterpret_cast<uint8_t*>(counters) + counters_bytes(pl.qblocks * batch));
         zero_block = true;
@@ -1377,10 +1093,7 @@ int launch_prepared(const void* qprep, long long nq, const void* tprep, long lon
         P.out = out;
         P.out_split_stride = 0;
     }
-    // (timing experiment: HM_KEEP_FLOORS=1 leaves the row thresholds of the previous launch in place -- "perfect"
-    // thresholds from the first tile on; results stay exact only when the same query runs again)
-    static const bool keep_floors = getenv("HM_KEEP_FLOORS") != nullptr;
-    if (zero_block) HM_CUDA_CHECK(cudaMemsetAsync(counters, 0, keep_floors ? counters_bytes(pl.qblocks * batch) : cbytes, stream));
+    if (zero_block) HM_CUDA_CHECK(cudaMemsetAsync(counters, 0, cbytes, stream));
     if (pl.qblocks > 0x7FFFFFFFll || pl.splits > 65535 || batch > 65535) {
         set_error("grid too large");
         return HM_ERR_UNSUPPORTED;
@@ -1405,45 +1118,6 @@ int launch_prepared(const void* qprep, long long nq, const void* tprep, long lon
         return HM_ERR_CUDA;
     }
     HM_CUDA_CHECK(cudaGetLastError());
-    if (trace_path) {   // development aid: dump the per-tile time stamps of CTA 0
-        static long long host[kTraceTiles * kTraceSlots];
-        HM_CUDA_CHECK(cudaStreamSynchronize(stream));
-        HM_CUDA_CHECK(cudaMemcpy(host, P.trace, sizeof(host), cudaMemcpyDeviceToHost));
-        {   // per-CTA records: <trace path>.ctas
-            const size_t nctas = (size_t)pl.qblocks * pl.splits * batch;
-            long long* rec = (long long*)malloc(nctas * kCtaSlots * sizeof(long long));
-            if (rec && cudaMemcpy(rec, P.trace + kTraceTiles * kTraceSlots, nctas * kCtaSlots * sizeof(long long), cudaMemcpyDeviceToHost) == cudaSuccess) {
-                char path[1024];
-                snprintf(path, sizeof(path), "%s.ctas", trace_path);
-                if (FILE* f = fopen(path, "w")) {
-                    fprintf(f, "# cta entry_ns prologue_done loop_done final_barrier exit tile8 tile32 tile64 tile192 smid slow_warp_chunks_lb slow_lane_chunks (globaltimer ns since the first entry); grid=(%lld,%d,%d)\n", pl.qblocks, pl.splits, batch);
-                    long long t0 = -1;
-                    for (size_t c = 0; c < nctas; ++c) if (rec[c * kCtaSlots] && (t0 < 0 || rec[c * kCtaSlots] < t0)) t0 = rec[c * kCtaSlots];
-                    for (size_t c = 0; c < nctas; ++c) {
-                        fprintf(f, "%zu", c);
-                        for (int k = 0; k < 9; ++k) fprintf(f, " %lld", rec[c * kCtaSlots + k] ? rec[c * kCtaSlots + k] - t0 : -1);
-                        fprintf(f, " %lld %lld %lld", rec[c * kCtaSlots + 11], rec[c * kCtaSlots + 9], rec[c * kCtaSlots + 10]);
-                        for (int k = 0; k < 9; ++k) fprintf(f, " %lld", rec[c * kCtaSlots + 12 + k] ? rec[c * kCtaSlots + 12 + k] - rec[c * kCtaSlots + 12] : -1);
-                        fprintf(f, "\n");
-                    }
-                    fclose(f);
-                }
-            }
-            free(rec);
-        }
-        cudaFree(P.trace);
-        if (FILE* f = fopen(trace_path, "w")) {
-            fprintf(f, "# tile producer_issue issuer_ready (unused) epi2_full epi2_scanned epi9_full issuer_unit1_free issuer_loop_top (cycles since first stamp); tiles/CTA=%d splits=%d cluster=%d core=%s\n",
-                    pl.tiles_per_split, pl.splits, pl.cluster, C::kScales ? "mxf4" : "i8");
-            long long t0 = host[0];
-            for (int i = 0; i < kTraceTiles; ++i) {
-                fprintf(f, "%d", i + P.trace_first);
-                for (int k = 0; k < 8; ++k) fprintf(f, " %lld", host[i * kTraceSlots + k] ? host[i * kTraceSlots + k] - t0 : -1);
-                fprintf(f, "\n");
-            }
-            fclose(f);
-        }
-    }
     if (keep_partials) {
         if (out_partials) *out_partials = partials;
         if (out_groups) *out_groups = pl.splits;
@@ -1586,7 +1260,7 @@ template <class C>
 static void describe_of(long long nq, long long nt, int batch, int sm_count, bool top1, char* buf, size_t n)
 {
     const TcPlan pl = plan_tc<C>(nq, nt, batch, sm_count);
-    const bool floor = !top1 && pl.splits > 1 && pl.tiles_per_split <= floor_max_tiles();
+    const bool floor = !top1 && pl.splits > 1;
     snprintf(buf, n, "hm_%s_knn%s%s_kernel grid=(%lld,%d,%d) cluster=%d tiles_per_cta=%d", C::kScales ? "f4" : "i8",
              top1 ? "1" : "2", floor ? "_floor" : "", pl.qblocks, pl.splits, batch, pl.cluster, pl.tiles_per_split);
 }

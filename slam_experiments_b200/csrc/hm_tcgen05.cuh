@@ -9,14 +9,6 @@
 namespace hm {
 namespace ptx {
 
-// experiment knob: suspend-time hint (ns) of mbarrier.try_wait -- a waiting thread sleeps in hardware up to this long
-// before the instruction returns false, instead of coming back to spin
-#ifndef HM_TRYWAIT_HINT_NS
-#define HM_TRYWAIT_HINT_NS 0
-#endif
-#define HM_STR2(x) #x
-#define HM_STR(x) HM_STR2(x)
-
 __device__ __forceinline__ uint32_t smem_u32(const void* p)
 {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));
@@ -63,11 +55,7 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity)
     asm volatile(
         "{\n\t"
         ".reg .pred P;\n\t"
-#if HM_TRYWAIT_HINT_NS
-        "mbarrier.try_wait.parity.shared::cta.b64 P, [%1], %2, " HM_STR(HM_TRYWAIT_HINT_NS) ";\n\t"
-#else
         "mbarrier.try_wait.parity.shared::cta.b64 P, [%1], %2;\n\t"
-#endif
         "selp.b32 %0, 1, 0, P;\n\t"
         "}\n"
         : "=r"(ok)
@@ -83,11 +71,7 @@ __device__ __forceinline__ bool mbar_try_wait_addr(uint32_t bar_addr, uint32_t p
     asm volatile(
         "{\n\t"
         ".reg .pred P;\n\t"
-#if HM_TRYWAIT_HINT_NS
-        "mbarrier.try_wait.parity.shared::cta.b64 P, [%1], %2, " HM_STR(HM_TRYWAIT_HINT_NS) ";\n\t"
-#else
         "mbarrier.try_wait.parity.shared::cta.b64 P, [%1], %2;\n\t"
-#endif
         "selp.b32 %0, 1, 0, P;\n\t"
         "}\n"
         : "=r"(ok)
@@ -232,21 +216,6 @@ __device__ __forceinline__ void mma_mxf4_ss(uint32_t tmem_d, uint64_t desc_a, ui
         : "memory");
 }
 
-// the same with the A operand read from TENSOR MEMORY (lane = row, 8 e2m1 elements per 32-bit column, 8 columns per
-// K = 64 instruction): no shared-memory reads for A
-__device__ __forceinline__ void mma_mxf4_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc,
-                                            uint32_t tmem_sfa, uint32_t tmem_sfb, uint32_t accumulate)
-{
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::mxf4.block_scale.block32 [%0], [%1], %2, %3, [%5], [%6], p;\n\t"
-        "}\n" ::"r"(tmem_d),
-        "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate), "r"(tmem_sfa), "r"(tmem_sfb)
-        : "memory");
-}
-
 // 32 lanes x 32 consecutive 32-bit columns, registers -> TMEM (scale-factor fill)
 __device__ __forceinline__ void tmem_st_32x32(uint32_t taddr, const uint32_t (&r)[32])
 {
@@ -286,17 +255,6 @@ __device__ __forceinline__ void tmem_ld_32x64(uint32_t taddr, uint32_t (&r)[64])
         "tcgen05.ld.sync.aligned.32x32b.x64.b32 "
         "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32, %33, %34, %35, %36, %37, %38, %39, %40, %41, %42, %43, %44, %45, %46, %47, %48, %49, %50, %51, %52, %53, %54, %55, %56, %57, %58, %59, %60, %61, %62, %63}, [%64];\n"
         : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31]), "=r"(r[32]), "=r"(r[33]), "=r"(r[34]), "=r"(r[35]), "=r"(r[36]), "=r"(r[37]), "=r"(r[38]), "=r"(r[39]), "=r"(r[40]), "=r"(r[41]), "=r"(r[42]), "=r"(r[43]), "=r"(r[44]), "=r"(r[45]), "=r"(r[46]), "=r"(r[47]), "=r"(r[48]), "=r"(r[49]), "=r"(r[50]), "=r"(r[51]), "=r"(r[52]), "=r"(r[53]), "=r"(r[54]), "=r"(r[55]), "=r"(r[56]), "=r"(r[57]), "=r"(r[58]), "=r"(r[59]), "=r"(r[60]), "=r"(r[61]), "=r"(r[62]), "=r"(r[63])
-        : "r"(taddr)
-        : "memory");
-}
-
-// 32 lanes x 16 consecutive 32-bit columns
-__device__ __forceinline__ void tmem_ld_32x16(uint32_t taddr, uint32_t (&r)[16])
-{
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];\n"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
         : "r"(taddr)
         : "memory");
 }

@@ -1,5 +1,5 @@
 """Development aid: wall time of one hm_match_host call from Python over small square problems (the single-launch path of
-csrc/hm_small.cu; HM_NO_SMALL_KERNEL=1 times the multi-launch / CUDA-graph path instead)."""
+csrc/hm_small.cu)."""
 import os
 import sys, time, numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))

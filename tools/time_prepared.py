@@ -12,7 +12,7 @@ q_host = synth.matchable_queries(t_host, nq, 3) if os.environ.get("HM_TP_DIST") 
 q = torch.from_numpy(q_host).cuda()
 t = torch.from_numpy(t_host).cuda()
 tp, qp = nat.prepare(t, variant=v), nat.prepare(q, variant=v)
-# sanity of an experiment build (timing-only builds with HM_TC_EXPERIMENT are wrong on purpose): tensor core == POPC
+# sanity check of the library under test: tensor core == POPC on a slice
 cq, ct = q[:1000], t[:50000]
 same = torch.equal(nat.knn2_keys(cq, ct, variant=v), nat.knn2_keys(cq, ct, variant="popc"))
 for _ in range(3):
