@@ -208,6 +208,33 @@ HM_API int hm_filter_matches(const uint64_t* fwd_keys, int64_t nq, const uint64_
                              int32_t* out_q, int32_t* out_t, int32_t* out_d, int32_t* out_count,
                              void* stream);
 
+/* ---- keyframe database: Lowe ratio test + database-wide mutual check over the global top-2 ---------------------
+ * keys[nq][2] are the GLOBAL top-2 keys of a query batch over the whole (possibly sharded) database, as
+ * hm_knn2_resident / hm_merge_top2 / the fused exchange return them (trainIdx = global row).
+ *
+ * hm_db_mutual_flags: the mutual check for ONE shard, the rows [row_lo, row_lo + shard_rows) held packed in
+ * shard_bits (shard_rows rows, t_stride bytes apart).  For every query q whose best row t1 = keys[q][0] lies in this
+ * range (and, with HM_FLAG_RATIO, that passes the ratio test), the nearest query of row t1 over all nq rows of `query`
+ * is computed (lowest query index on ties); out_flags[q] = 1 iff that is q.  Every other entry of out_flags[nq] is
+ * written 0, including queries whose t1 another shard owns, so the element-wise MAX over the shards' flags is the
+ * database-wide answer.  Work is a top-1 k-NN of at most nq gathered shard rows against the nq queries; with the
+ * kind::mxf4 core (HM_VARIANT_F4, or AUTO when it resolves to it for nq x nq) only the rows this shard owns are
+ * computed, the count of which stays on the device.  Nothing is proportional to the database size: the workspace is
+ * hm_db_mutual_workspace_bytes(nq, variant).  flags: HM_FLAG_RATIO and HM_FLAG_MUTUAL only.
+ *
+ * hm_db_filter: ratio test (HM_FLAG_RATIO) and mutual check (HM_FLAG_MUTUAL: keep q iff mutual_flags[q] != 0) on the
+ * global keys, then the ordered compaction: out_q / out_t / out_d[nq] (queryIdx, global row, distance) ordered by
+ * queryIdx, *out_count matches.  mutual_flags may be NULL only without HM_FLAG_MUTUAL; with neither flag every query
+ * keeps its best row (knnMatch k=1). */
+HM_API size_t hm_db_mutual_workspace_bytes(int64_t nq, int variant);
+HM_API int hm_db_mutual_flags(const uint64_t* keys, int64_t nq, const uint8_t* query, int64_t q_stride,
+                              const uint8_t* shard_bits, int64_t shard_rows, int64_t t_stride, uint64_t row_lo,
+                              unsigned flags, const uint16_t* ratio_lut_host, uint8_t* out_flags,
+                              int variant, void* workspace, size_t workspace_bytes, void* stream);
+HM_API int hm_db_filter(const uint64_t* keys, int64_t nq, const uint8_t* mutual_flags, unsigned flags,
+                        const uint16_t* ratio_lut_host, int32_t* out_q, int32_t* out_t, int32_t* out_d,
+                        int32_t* out_count, void* stream);
+
 /* knn2 (+ the swapped pass when HM_FLAG_MUTUAL) + hm_filter_matches in one enqueue.
  * out_keys (fwd, [batch][nq][2]) may be NULL when the caller only wants the match list.
  * With the kind::mxf4 core the forward k-NN kernel applies the ratio test to each row's final keys itself and marks the

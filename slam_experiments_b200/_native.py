@@ -36,6 +36,7 @@ EXPORTS = (
     "hm_knn2", "hm_knn2_batched", "hm_default_tensor_variant", "hm_prepared_bytes", "hm_prepared_workspace_bytes", "hm_prepare", "hm_knn2_prepared", "hm_knn2_prepared_partials", "hm_knn2_prepared_exchange",
     "hm_resident_workspace_bytes", "hm_knn2_resident", "hm_knn2_resident_exchange",
     "hm_merge_top2", "hm_exchange_bytes", "hm_exchange_merge", "hm_filter_matches", "hm_match_fused", "hm_gather_points", "hm_rasterize_mask",
+    "hm_db_mutual_workspace_bytes", "hm_db_mutual_flags", "hm_db_filter",
     "hm_context_create", "hm_context_destroy", "hm_knn2_host", "hm_match_host", "hm_frame_put", "hm_frame_match",
     "hm_resident_query_begin", "hm_resident_query_end",
     "hm_orb_workspace_bytes", "hm_orb_level_geometry", "hm_orb_angles_to_cs", "hm_orb_build_pyramid", "hm_orb_describe",
@@ -99,6 +100,12 @@ def _declare(L):
     L.hm_match_fused.restype = ci
     L.hm_match_fused.argtypes = [vp, i64, i64, i64, vp, i64, i64, i64, ci, cu, vp, c.c_double,
                                  vp, vp, vp, vp, vp, ci, vp, sz, vp]
+    L.hm_db_mutual_workspace_bytes.restype = sz
+    L.hm_db_mutual_workspace_bytes.argtypes = [i64, ci]
+    L.hm_db_mutual_flags.restype = ci
+    L.hm_db_mutual_flags.argtypes = [vp, i64, vp, i64, vp, i64, i64, u64, cu, vp, vp, ci, vp, sz, vp]
+    L.hm_db_filter.restype = ci
+    L.hm_db_filter.argtypes = [vp, i64, vp, cu, vp, vp, vp, vp, vp, vp]
     L.hm_gather_points.restype = ci
     L.hm_gather_points.argtypes = [vp, vp, vp, i64, ci, vp, i64, vp, i64, vp, vp, vp]
     L.hm_rasterize_mask.restype = ci
@@ -493,6 +500,65 @@ def match_fused(query: torch.Tensor, train: torch.Tensor, ratio: Optional[float]
                                _stream_ptr(dev)), "hm_match_fused")
     del lut
     return (oq, ot, od, cnt, keys) if want_keys else (oq, ot, od, cnt)
+
+
+def _check_keys(keys: torch.Tensor) -> None:
+    if keys.dtype != torch.int64 or keys.dim() != 2 or keys.shape[1] != 2 or not keys.is_cuda or not keys.is_contiguous():
+        raise ValueError("keys must be a contiguous CUDA int64 tensor [Nq, 2]")
+
+
+def db_mutual_workspace_bytes(nq: int, variant="auto") -> int:
+    return int(lib().hm_db_mutual_workspace_bytes(nq, variant_id(variant)))
+
+
+def db_mutual_flags(keys: torch.Tensor, query: torch.Tensor, shard_bits: torch.Tensor, row_lo: int,
+                    ratio: Optional[float] = None, variant="auto", out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """``hm_db_mutual_flags``: ``uint8 [Nq]`` mutual flags of one shard of a keyframe database.
+
+    ``keys`` are the global top-2 keys of ``query`` over the whole database; ``shard_bits`` holds the database rows
+    ``[row_lo, row_lo + len(shard_bits))``.  ``flags[q] = 1`` iff the best row of ``q`` lies in this shard (and passes
+    the ratio test when ``ratio`` is given) and ``q`` is the lowest-index nearest query of that row; every other entry
+    is 0, so the element-wise maximum over all shards is the database-wide mutual check."""
+    _check_keys(keys)
+    _check_desc(query, "query")
+    _check_desc(shard_bits, "shard_bits")
+    nq, rows = query.shape[0], shard_bits.shape[0]
+    if keys.shape[0] != nq:
+        raise ValueError("keys and query differ in rows")
+    dev = query.device
+    if out is None:
+        out = torch.empty(nq, dtype=torch.uint8, device=dev)
+    flags, lut = (FLAG_MUTUAL | FLAG_RATIO, _ratio_lut_cached(float(ratio))) if ratio is not None else (FLAG_MUTUAL, None)
+    v = variant_id(variant)
+    L = lib()
+    with on_device(dev):
+        ws = workspace(L.hm_db_mutual_workspace_bytes(nq, v), dev)
+        check(L.hm_db_mutual_flags(keys.data_ptr(), nq, query.data_ptr(), query.stride(0) if nq else DESC_BYTES,
+                                   shard_bits.data_ptr(), rows, shard_bits.stride(0) if rows else DESC_BYTES, row_lo,
+                                   flags, lut.ctypes.data if lut is not None else None, out.data_ptr(), v,
+                                   ws.data_ptr(), ws.numel(), _stream_ptr(dev)), "hm_db_mutual_flags")
+    return out
+
+
+def db_filter(keys: torch.Tensor, mutual_flags: Optional[torch.Tensor] = None, ratio: Optional[float] = None):
+    """``hm_db_filter``: ratio test and (with ``mutual_flags``) the mutual check on global top-2 keys, compacted in
+    query order.  Returns ``(q, t, d, count)`` device tensors: ``q / t / d [Nq] int32`` (queryIdx, global database row,
+    distance), valid up to ``count [1]``."""
+    _check_keys(keys)
+    nq = keys.shape[0]
+    dev = keys.device
+    flags, lut = (FLAG_RATIO, _ratio_lut_cached(float(ratio))) if ratio is not None else (0, None)
+    if mutual_flags is not None:
+        if mutual_flags.dtype != torch.uint8 or not mutual_flags.is_cuda or mutual_flags.numel() < nq:
+            raise ValueError("mutual_flags must be a CUDA uint8 tensor of at least Nq entries")
+        flags |= FLAG_MUTUAL
+    out = torch.empty((3, nq), dtype=torch.int32, device=dev)
+    cnt = torch.empty(1, dtype=torch.int32, device=dev)
+    with on_device(dev):
+        check(lib().hm_db_filter(keys.data_ptr(), nq, mutual_flags.data_ptr() if mutual_flags is not None else None, flags,
+                                 lut.ctypes.data if lut is not None else None, out[0].data_ptr(), out[1].data_ptr(),
+                                 out[2].data_ptr(), cnt.data_ptr(), _stream_ptr(dev)), "hm_db_filter")
+    return out[0], out[1], out[2], cnt
 
 
 def gather_points(q_idx: torch.Tensor, t_idx: torch.Tensor, count: torch.Tensor, query_pts: torch.Tensor,

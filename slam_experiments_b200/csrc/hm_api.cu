@@ -591,6 +591,110 @@ HM_API int hm_match_fused(const uint8_t* query, int64_t nq, int64_t q_stride, in
     return launch_filter(fwd, nq, bwd, nt, batch, flags, lut, thr, out_q, out_t, out_d, out_count, st);
 }
 
+// ---- keyframe database: ratio test + database-wide mutual check ----------------------------------------------------
+// Workspace of hm_db_mutual_flags, all sized by the query batch alone: [count | list nq | owner nq | best nq x 2 |
+// gathered rows nq x 32 | k-NN scratch of the nq x nq top-1 pass].  `v` is the variant resolved for nq x nq.
+struct DbMutualLayout {
+    size_t list, owner, best, gathered, knn, total;
+};
+
+static DbMutualLayout db_mutual_layout(long long nq, int v, int sm)
+{
+    DbMutualLayout L;
+    L.list = 256;
+    L.owner = L.list + align_up((size_t)nq * 4);
+    L.best = L.owner + align_up((size_t)nq * 4);
+    L.gathered = L.best + align_up((size_t)nq * 16);
+    L.knn = L.gathered + align_up((size_t)nq * HM_DESC_BYTES);
+    // kind::mxf4 runs the candidate pass (the kernel gathers the rows through the list); the other cores a dense pass
+    // over the gathered rows
+    const size_t k = v == HM_VARIANT_F4 ? tc_workspace_bytes(nq, nq, 1, sm, true, HM_VARIANT_F4) : knn_workspace(nq, nq, 1, v, sm);
+    L.total = L.knn + align_up(k) + 256;
+    return L;
+}
+
+HM_API size_t hm_db_mutual_workspace_bytes(int64_t nq, int variant)
+{
+    DeviceInfo di;
+    int sm = 148;   // sizing only; B200
+    if (device_info(&di) == HM_OK) sm = di.sm_count;
+    if (nq < 0 || variant < HM_VARIANT_AUTO || variant > HM_VARIANT_F4) return 0;
+    if (nq == 0) return 256;
+    return db_mutual_layout(nq, resolve_variant(variant, nq, nq, 1), sm).total;
+}
+
+HM_API int hm_db_mutual_flags(const uint64_t* keys, int64_t nq, const uint8_t* query, int64_t q_stride,
+                              const uint8_t* shard_bits, int64_t shard_rows, int64_t t_stride, uint64_t row_lo,
+                              unsigned flags, const uint16_t* ratio_lut_host, uint8_t* out_flags, int variant,
+                              void* workspace, size_t workspace_bytes, void* stream)
+{
+    DeviceInfo di;
+    int rc = device_info(&di);
+    if (rc != HM_OK) return rc;
+    if (nq < 0 || shard_rows < 0 || (nq > 0 && (!keys || !out_flags)) || (flags & ~(HM_FLAG_RATIO | HM_FLAG_MUTUAL)) ||
+        variant < HM_VARIANT_AUTO || variant > HM_VARIANT_F4 || row_lo + (uint64_t)shard_rows > 0xFFFFFFFFull) {
+        set_error("hm_db_mutual_flags: bad arguments");
+        return HM_ERR_INVALID_ARGUMENT;
+    }
+    if (nq == 0) return HM_OK;
+    if ((rc = check_rows(query, nq, q_stride, "query")) != HM_OK) return rc;
+    if ((rc = check_rows(shard_bits, shard_rows, t_stride, "shard_bits")) != HM_OK) return rc;
+    RatioLut lut;
+    int thr;
+    if ((rc = build_filter_args(flags & HM_FLAG_RATIO, ratio_lut_host, 0.0, &lut, &thr)) != HM_OK) return rc;
+    const int v = resolve_variant(variant, nq, nq, 1);
+    const DbMutualLayout L = db_mutual_layout(nq, v, di.sm_count);
+    if (!workspace || workspace_bytes < L.total || (reinterpret_cast<uintptr_t>(workspace) & 255)) {
+        set_error("workspace too small or misaligned: need %zu bytes, 256-byte aligned, got %zu", L.total, workspace_bytes);
+        return HM_ERR_WORKSPACE;
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    uint8_t* ws = static_cast<uint8_t*>(workspace);
+    int* count = reinterpret_cast<int*>(ws);
+    int* list = reinterpret_cast<int*>(ws + L.list);
+    int* owner = reinterpret_cast<int*>(ws + L.owner);
+    unsigned long long* best = reinterpret_cast<unsigned long long*>(ws + L.best);
+    uint8_t* gathered = v == HM_VARIANT_F4 ? nullptr : ws + L.gathered;
+    unsigned char* fl = reinterpret_cast<unsigned char*>(out_flags);
+    const unsigned long long* k = reinterpret_cast<const unsigned long long*>(keys);
+    // every flag is written (0) here, also on a shard without rows: the MAX over the shards needs each one's zeros
+    if ((rc = launch_db_select(k, nq, row_lo, row_lo + (uint64_t)shard_rows, (flags & HM_FLAG_RATIO) ? 1 : 0, lut,
+                               shard_bits, t_stride, list, owner, count, gathered, fl, st)) != HM_OK)
+        return rc;
+    if (shard_rows == 0) return HM_OK;
+    // top-1 over the query batch of every listed shard row: "query" side = shard rows, "train" side = the batch
+    KnnProblem r{};
+    r.q = gathered ? gathered : shard_bits; r.nq = nq; r.q_stride = gathered ? HM_DESC_BYTES : t_stride;
+    r.t = query; r.nt = nq; r.t_stride = q_stride;
+    r.batch = 1; r.top1 = true;
+    uint8_t* knn_ws = ws + L.knn;
+    const size_t knn_bytes = L.total - L.knn;
+    if (v == HM_VARIANT_F4) rc = launch_tc_knn1_candidates(r, list, count, best, knn_ws, knn_bytes, di.sm_count, st);
+    else                    rc = knn2_dispatch(r, best, v, knn_ws, knn_bytes, st);
+    if (rc != HM_OK) return rc;
+    return launch_db_resolve(owner, count, best, nq, fl, st);
+}
+
+HM_API int hm_db_filter(const uint64_t* keys, int64_t nq, const uint8_t* mutual_flags, unsigned flags,
+                        const uint16_t* ratio_lut_host, int32_t* out_q, int32_t* out_t, int32_t* out_d, int32_t* out_count,
+                        void* stream)
+{
+    DeviceInfo di;
+    int rc = device_info(&di);
+    if (rc != HM_OK) return rc;
+    if (nq < 0 || !out_count || (nq > 0 && (!keys || !out_q || !out_t || !out_d)) ||
+        (flags & ~(HM_FLAG_RATIO | HM_FLAG_MUTUAL)) || ((flags & HM_FLAG_MUTUAL) && nq > 0 && !mutual_flags)) {
+        set_error("hm_db_filter: bad arguments");
+        return HM_ERR_INVALID_ARGUMENT;
+    }
+    RatioLut lut;
+    int thr;
+    if ((rc = build_filter_args(flags, ratio_lut_host, 0.0, &lut, &thr)) != HM_OK) return rc;
+    return launch_filter(reinterpret_cast<const unsigned long long*>(keys), nq, nullptr, 0, 1, flags, lut, thr, out_q,
+                         out_t, out_d, out_count, static_cast<cudaStream_t>(stream), nullptr,
+                         reinterpret_cast<const unsigned char*>(mutual_flags));
+}
+
 HM_API int hm_gather_points(const int32_t* q_idx, const int32_t* t_idx, const int32_t* count, int64_t stride, int batch,
                             const int32_t* query_pts, int64_t nq, const int32_t* train_pts, int64_t nt,
                             int32_t* out_query_pts, int32_t* out_train_pts, void* stream)

@@ -273,10 +273,22 @@ int launch_exchange_merge(const unsigned long long* local_keys, int local_groups
                           void* const* peers, long long max_rows, unsigned epoch, unsigned long long* out,
                           cudaStream_t stream);
 
-// slot_of != null: bwd holds one entry per CANDIDATE train row (SelectArgs), train row t at slot_of[t] - 1
+// slot_of != null: bwd holds one entry per CANDIDATE train row (SelectArgs), train row t at slot_of[t] - 1;
+// mutual_flags != null: the mutual check reads mutual_flags[b][q] instead of bwd (keyframe database, hm_db_filter)
 int launch_filter(const unsigned long long* fwd, long long nq, const unsigned long long* bwd, long long nt,
                   int batch, unsigned flags, const RatioLut& lut, int thr_ceil, int* out_q, int* out_t,
-                  int* out_d, int* out_count, cudaStream_t stream, const int* slot_of = nullptr);
+                  int* out_d, int* out_count, cudaStream_t stream, const int* slot_of = nullptr,
+                  const unsigned char* mutual_flags = nullptr);
+
+// keyframe-database mutual check, one shard (hm_db_mutual_flags).  select: flags[0 .. nq) = 0 and the ordered list of
+// the queries whose best row lies in [row_lo, row_hi) (and pass the ratio test when use_ratio): list[s] = local shard
+// row, owner[s] = query, *count = entries; with `gathered` != null also gathered[s] = the shard row's 32 bytes (rows
+// past *count zeroed).  resolve: flags[owner[s]] = 1 iff best[s] (top-1 key over the queries) names owner[s].
+int launch_db_select(const unsigned long long* keys, long long nq, unsigned long long row_lo, unsigned long long row_hi,
+                     int use_ratio, const RatioLut& lut, const uint8_t* shard_bits, long long t_stride, int* list,
+                     int* owner, int* count, uint8_t* gathered, unsigned char* flags, cudaStream_t stream);
+int launch_db_resolve(const int* owner, const int* count, const unsigned long long* best, long long nq,
+                      unsigned char* flags, cudaStream_t stream);
 
 void describe_tc_launch(long long nq, long long nt, int batch, int sm_count, int variant, bool top1, char* buf, size_t n);
 int launch_gather_points(const int* q_idx, const int* t_idx, const int* count, long long stride, int batch,

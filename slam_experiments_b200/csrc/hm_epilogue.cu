@@ -62,8 +62,29 @@ struct FilterParams {
     int* out_d;
     int* out_count;
     const int* slot_of;              // [batch][nt] candidate slots + 1 (SelectArgs), null = bwd indexed by train row
+    const unsigned char* mutual;     // [batch][nq] per-query mutual flags (keyframe database), null = use bwd
     RatioLut lut;
 };
+
+// Ordered block scan of one flag per thread (all kFilterThreads threads call it): returns how many threads below this
+// one have `keep` set and, through `total`, how many in the CTA do.  warp_sums is shared scratch of 32 ints; the caller
+// synchronises before warp_sums is written again.
+__device__ __forceinline__ int ordered_scan(int keep, int* warp_sums, int& total)
+{
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const unsigned ballot = __ballot_sync(0xFFFFFFFFu, keep);
+    const int prefix = __popc(ballot & ((1u << lane) - 1));
+    if (lane == 0) warp_sums[wid] = __popc(ballot);
+    __syncthreads();
+    int v = lane < (kFilterThreads / 32) ? warp_sums[lane] : 0;
+    int incl = v;
+    for (int o = 1; o < 32; o <<= 1) {
+        int n = __shfl_up_sync(0xFFFFFFFFu, incl, o);
+        if (lane >= o) incl += n;
+    }
+    total = __shfl_sync(0xFFFFFFFFu, incl, 31);
+    return __shfl_sync(0xFFFFFFFFu, incl - v, wid) + prefix;
+}
 
 // One CTA per problem: rows are visited in order so the output stays sorted by queryIdx.
 __global__ void __launch_bounds__(kFilterThreads) hm_filter_kernel(const FilterParams P)
@@ -71,7 +92,7 @@ __global__ void __launch_bounds__(kFilterThreads) hm_filter_kernel(const FilterP
     __shared__ int warp_sums[32];
     __shared__ int s_base;
     __shared__ unsigned s_min;
-    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const int tid = threadIdx.x, lane = tid & 31;
     const int b = blockIdx.x;
     const unsigned long long* fwd = P.fwd + (long long)b * P.nq * 2;
     const unsigned long long* bwd = P.bwd ? P.bwd + (long long)b * P.nt * 2 : nullptr;
@@ -108,7 +129,9 @@ __global__ void __launch_bounds__(kFilterThreads) hm_filter_kernel(const FilterP
             if (keep && (P.flags & HM_FLAG_RATIO)) {
                 keep = (k.y != kNoMatch) && d1 < (int)P.lut.v[min((unsigned)(k.y >> 32), 256u)];
             }
-            if (keep && (P.flags & HM_FLAG_MUTUAL)) {
+            if (keep && (P.flags & HM_FLAG_MUTUAL) && P.mutual) {
+                keep = P.mutual[(long long)b * P.nq + r] != 0;
+            } else if (keep && (P.flags & HM_FLAG_MUTUAL)) {
                 // bwd is indexed by train row, or -- after the candidate pass -- by the row's candidate slot (a row
                 // that reaches this line passed the ratio test, so the k-NN kernel gave its best train row a slot)
                 const long long slot = P.slot_of ? (long long)P.slot_of[(long long)b * P.nt + t1] - 1 : (long long)t1;
@@ -116,25 +139,11 @@ __global__ void __launch_bounds__(kFilterThreads) hm_filter_kernel(const FilterP
             }
             if (keep && (P.flags & HM_FLAG_DIST_THRESHOLD)) keep = d1 < limit;
         }
-        // ordered block scan of the keep flags
-        const unsigned ballot = __ballot_sync(0xFFFFFFFFu, keep);
-        const int prefix = __popc(ballot & ((1u << lane) - 1));
-        if (lane == 0) warp_sums[wid] = __popc(ballot);
-        __syncthreads();
-        int wbase = 0, total = 0;
-        {
-            int v = lane < (kFilterThreads / 32) ? warp_sums[lane] : 0;
-            int incl = v;
-            for (int o = 1; o < 32; o <<= 1) {
-                int n = __shfl_up_sync(0xFFFFFFFFu, incl, o);
-                if (lane >= o) incl += n;
-            }
-            wbase = __shfl_sync(0xFFFFFFFFu, incl - v, wid);
-            total = __shfl_sync(0xFFFFFFFFu, incl, 31);
-        }
+        int total;
+        const int offset = ordered_scan(keep, warp_sums, total);
         const int base = s_base;
         if (keep) {
-            const int pos = base + wbase + prefix;
+            const int pos = base + offset;
             oq[pos] = (int)r;
             ot[pos] = t1;
             od[pos] = d1;
@@ -144,6 +153,87 @@ __global__ void __launch_bounds__(kFilterThreads) hm_filter_kernel(const FilterP
         __syncthreads();
     }
     if (tid == 0) P.out_count[b] = s_base;
+}
+
+// ---- keyframe database: mutual check of one shard (hm_db_mutual_flags) -------------------------------------------
+// The mutual check asks, for the best database row t1 of every query, which query of the batch is nearest to t1.  The
+// shard that holds t1 answers: select lists its queries in query order (one CTA, the filter's ordered scan), a top-1
+// k-NN of the listed shard rows against the query batch follows (hm_api.cu), and resolve marks each listed query that
+// is its row's nearest query.  A row named by several queries is listed once per query: an extra row of an nq-row pass
+// costs less than a table indexed by database row.
+struct DbSelectParams {
+    const unsigned long long* keys;  // [nq][2] global top-2
+    long long nq;
+    unsigned long long row_lo, row_hi;
+    int use_ratio;
+    const uint8_t* shard_bits;
+    long long t_stride;
+    int* list;                       // [nq] local shard rows
+    int* owner;                      // [nq] the query that named each row
+    int* count;
+    uint8_t* gathered;               // [nq][32] or null (the kind::mxf4 k-NN kernel gathers through `list` itself)
+    unsigned char* flags;            // [nq]
+    RatioLut lut;
+};
+
+__global__ void __launch_bounds__(kFilterThreads) hm_db_select_kernel(const DbSelectParams P)
+{
+    __shared__ int warp_sums[32];
+    __shared__ int s_base;
+    const int tid = threadIdx.x;
+    if (tid == 0) s_base = 0;
+    __syncthreads();
+    for (long long r0 = 0; r0 < P.nq; r0 += kFilterThreads) {
+        const long long r = r0 + tid;
+        int own = 0;
+        unsigned long long t1 = 0;
+        if (r < P.nq) {
+            const ulonglong2 k = *reinterpret_cast<const ulonglong2*>(P.keys + r * 2);
+            t1 = k.x & 0xFFFFFFFFull;
+            own = k.x != kNoMatch && t1 >= P.row_lo && t1 < P.row_hi;
+            if (own && P.use_ratio)     // the filter's ratio test: a row it drops needs no backward answer
+                own = k.y != kNoMatch && (unsigned)(k.x >> 32) < (unsigned)P.lut.v[min((unsigned)(k.y >> 32), 256u)];
+            P.flags[r] = 0;
+        }
+        int total;
+        const int offset = ordered_scan(own, warp_sums, total);
+        const int base = s_base;
+        if (own) {
+            const int s = base + offset;
+            const long long local = (long long)(t1 - P.row_lo);
+            P.list[s] = (int)local;
+            P.owner[s] = (int)r;
+            if (P.gathered) {
+                const uint4* src = reinterpret_cast<const uint4*>(P.shard_bits + local * P.t_stride);
+                uint4* dst = reinterpret_cast<uint4*>(P.gathered + (long long)s * HM_DESC_BYTES);
+                dst[0] = src[0];
+                dst[1] = src[1];
+            }
+        }
+        __syncthreads();
+        if (tid == 0) s_base = base + total;
+        __syncthreads();
+    }
+    const int n = s_base;
+    if (tid == 0) *P.count = n;
+    if (P.gathered) {                // the dense k-NN pass reads all nq rows: keep the unused ones defined
+        for (long long s = n + tid; s < P.nq; s += kFilterThreads) {
+            uint4* dst = reinterpret_cast<uint4*>(P.gathered + s * HM_DESC_BYTES);
+            dst[0] = make_uint4(0, 0, 0, 0);
+            dst[1] = make_uint4(0, 0, 0, 0);
+        }
+    }
+}
+
+__global__ void __launch_bounds__(256) hm_db_resolve_kernel(const int* __restrict__ owner, const int* __restrict__ count,
+                                                            const unsigned long long* __restrict__ best,
+                                                            unsigned char* __restrict__ flags)
+{
+    const int s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= *count) return;
+    const int q = owner[s];
+    const unsigned long long k = best[(long long)s * 2];
+    if (k != kNoMatch && (long long)(k & 0xFFFFFFFFull) == q) flags[q] = 1;
 }
 
 }  // namespace
@@ -206,16 +296,42 @@ int launch_exchange_merge(const unsigned long long* local_keys, int local_groups
 
 int launch_filter(const unsigned long long* fwd, long long nq, const unsigned long long* bwd, long long nt,
                   int batch, unsigned flags, const RatioLut& lut, int thr_ceil, int* out_q, int* out_t,
-                  int* out_d, int* out_count, cudaStream_t stream, const int* slot_of)
+                  int* out_d, int* out_count, cudaStream_t stream, const int* slot_of,
+                  const unsigned char* mutual_flags)
 {
     if (batch <= 0) return HM_OK;
     FilterParams P{};
     P.slot_of = slot_of;
+    P.mutual = mutual_flags;
     P.fwd = fwd; P.bwd = bwd; P.nq = nq; P.nt = nt; P.flags = flags;
     P.out_q = out_q; P.out_t = out_t; P.out_d = out_d; P.out_count = out_count;
     P.lut = lut;
     P.thr_ceil = thr_ceil;
     hm_filter_kernel<<<batch, kFilterThreads, 0, stream>>>(P);
+    HM_CUDA_CHECK(cudaGetLastError());
+    return HM_OK;
+}
+
+int launch_db_select(const unsigned long long* keys, long long nq, unsigned long long row_lo, unsigned long long row_hi,
+                     int use_ratio, const RatioLut& lut, const uint8_t* shard_bits, long long t_stride, int* list,
+                     int* owner, int* count, uint8_t* gathered, unsigned char* flags, cudaStream_t stream)
+{
+    if (nq <= 0) return HM_OK;
+    DbSelectParams P{};
+    P.keys = keys; P.nq = nq; P.row_lo = row_lo; P.row_hi = row_hi; P.use_ratio = use_ratio;
+    P.shard_bits = shard_bits; P.t_stride = t_stride;
+    P.list = list; P.owner = owner; P.count = count; P.gathered = gathered; P.flags = flags;
+    P.lut = lut;
+    hm_db_select_kernel<<<1, kFilterThreads, 0, stream>>>(P);
+    HM_CUDA_CHECK(cudaGetLastError());
+    return HM_OK;
+}
+
+int launch_db_resolve(const int* owner, const int* count, const unsigned long long* best, long long nq,
+                      unsigned char* flags, cudaStream_t stream)
+{
+    if (nq <= 0) return HM_OK;
+    hm_db_resolve_kernel<<<(unsigned)ceil_div(nq, 256), 256, 0, stream>>>(owner, count, best, flags);
     HM_CUDA_CHECK(cudaGetLastError());
     return HM_OK;
 }

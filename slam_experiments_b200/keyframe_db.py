@@ -235,6 +235,26 @@ class NativeOps:
         with nat.on_device(self.device):
             return self._staging.to_host("keys", keys)
 
+    # ---- ratio test + database-wide mutual check over the global top-2 (all on torch's current stream) ----
+    def mutual_flags(self, keys: torch.Tensor, query: torch.Tensor, shard, row_lo: int,
+                     ratio: Optional[float]) -> torch.Tensor:
+        """This shard's mutual flags ``uint8 [Nq]``: 1 where the query's best row is held here and the query is that
+        row's nearest query; 0 everywhere else.  The top-1 pass over the query batch uses the shard's tensor core when
+        it has a prepared image (kind::mxf4 computes only the rows this shard owns), else the configured variant."""
+        variant = shard["tc"] if shard.get("prepared") is not None else self.variant
+        return nat.db_mutual_flags(keys, query, shard["bits"], row_lo, ratio, variant=variant)
+
+    def all_reduce_max(self, flags: torch.Tensor, group) -> torch.Tensor:
+        """Element-wise MAX of every rank's flags.  This is its own collective on the process group: it shares nothing
+        with the k-NN exchange (symmetric buffer, slots, epochs).  An empty batch still joins with one zero."""
+        import torch.distributed as dist
+        buf = flags if flags.numel() else torch.zeros(1, dtype=torch.uint8, device=self.device)
+        dist.all_reduce(buf, op=dist.ReduceOp.MAX, group=group)
+        return buf
+
+    def filter_matches(self, keys: torch.Tensor, flags: Optional[torch.Tensor], ratio: Optional[float]):
+        return nat.db_filter(keys, flags, ratio)
+
 
 class ShardedKeyframeDatabase:
     """Train collection sharded by contiguous keyframe ranges, one shard per rank.
@@ -339,6 +359,45 @@ class ShardedKeyframeDatabase:
         gidx, dist = gidx[:, :kk], dist[:, :kk]
         img, local = nat.locate_rows(self.starts, gidx)
         return img, local, dist
+
+    # ---- ratio test + mutual check over the whole database ---------------------------------------------
+    def match_device(self, query_dev: torch.Tensor, *, ratio: Optional[float] = None, cross_check: bool = False):
+        """knnMatch k=2 over the whole database, then Lowe's ratio test and the database-wide mutual check.
+
+        Returns device tensors ``(q, t, d, count)``: ``q / t / d [Nq] int32`` hold queryIdx, GLOBAL database row and
+        distance of the kept queries in query order, ``count [1]`` how many there are.  A query is kept iff
+        ``ratio`` is None or its two nearest rows satisfy ``d1 < ratio * d2`` (float64; a database of fewer than two rows
+        drops every query), and -- with ``cross_check`` -- it is the lowest-index nearest query of its best row among
+        the ``Nq`` queries of the batch.  Every rank calls it with the same arguments and gets the same list; with
+        ``world_size > 1`` and ``cross_check`` there is one MAX all-reduce over ``Nq`` bytes on the process group."""
+        nq = query_dev.shape[0]
+        keys = self.knn2_keys_device(query_dev) if nq else torch.empty((0, 2), dtype=torch.int64, device=query_dev.device)
+        flags = None
+        if cross_check:
+            flags = self.ops.mutual_flags(keys, query_dev, self.shard, self.row_lo, ratio)
+            if self.world_size > 1:
+                flags = self.ops.all_reduce_max(flags, self.group)
+        return self.ops.filter_matches(keys, flags, ratio)
+
+    def match_tensors(self, query, *, ratio: Optional[float] = None, cross_check: bool = False):
+        """``(queryIdx, imgIdx, trainIdx, distance)`` int32 arrays of :meth:`match_device`, ordered by queryIdx;
+        ``(imgIdx, trainIdx)`` locate the best row in the keyframe collection as :meth:`knn_tensors` does."""
+        q = np.asarray(query)
+        if q.size == 0:
+            q = np.empty((0, nat.DESC_BYTES), np.uint8)
+        if q.dtype != np.uint8 or q.ndim != 2 or q.shape[1] != nat.DESC_BYTES:
+            raise MatcherError("query: expected uint8 [N, 32] descriptors")
+        oq, ot, od, cnt = self.match_device(self.ops.upload(q), ratio=ratio, cross_check=cross_check)
+        host = self.ops.to_host(torch.cat([cnt.view(1), oq.view(-1), ot.view(-1), od.view(-1)]))   # one D2H
+        n, nq = int(host[0]), q.shape[0]
+        qi, gidx, d = host[1:1 + n], host[1 + nq:1 + nq + n], host[1 + 2 * nq:1 + 2 * nq + n]
+        img, local = nat.locate_rows(self.starts, gidx.astype(np.int64))
+        return qi.astype(np.int32), img, local, d.astype(np.int32)
+
+    def match(self, query, *, ratio: Optional[float] = None, cross_check: bool = False) -> tuple:
+        """The kept matches of :meth:`match_tensors` as a tuple of ``cv2.DMatch`` (``imgIdx`` = keyframe index)."""
+        qi, img, local, d = self.match_tensors(query, ratio=ratio, cross_check=cross_check)
+        return tuple(_build_dmatches(qi, local, d, img))
 
     def knnMatch(self, queryDescriptors, k: int = 2) -> tuple:
         """cv2 ``bf.knnMatch(query, k)`` over the whole (sharded) collection."""
