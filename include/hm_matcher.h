@@ -140,6 +140,44 @@ HM_API int hm_knn2_resident_exchange(const uint8_t* query, int64_t nq, int64_t q
                                      uint32_t epoch, uint64_t* out_keys, int variant, void* workspace,
                                      size_t workspace_bytes, void* stream);
 
+/* ---- keyframe database: search a selection of the train rows ------------------------------------------------------
+ * A selection is a list of n_runs RUNS [lo, hi) of train rows (shard-local), ascending, disjoint and non-empty, with
+ * hi <= nt < 2^32.  The result equals hm_knn2 over the concatenation of the selected rows, with every trainIdx mapped
+ * back to its row (+ train_base): the stable top-2 over the selected rows, ties to the lowest row.  Unselected rows
+ * cost nothing beyond the 128-row tiles a run starts or ends in.
+ *  runs_host[n_runs][2]  host array (lo, hi): validated (HM_ERR_INVALID_ARGUMENT before any launch for unsorted,
+ *                        overlapping, empty or out-of-range runs) and planned from
+ *  runs_dev[n_runs][4]   device array the caller uploads with the same runs: lo, hi, the 128-row tiles the runs before
+ *                        it touch (sum of ceil(hi / 128) - floor(lo / 128)) and the rows the runs before it hold
+ * n_runs == 0 selects nothing: out_keys is all HM_NO_MATCH (the _exchange entry needs n_runs >= 1; a rank without
+ * selected rows joins the exchange through hm_exchange_merge with HM_NO_MATCH keys).
+ *
+ * hm_knn2_resident_runs: over a prepared image (hm_prepare) -- the k-NN kernel walks the runs in place, one launch
+ * (kind::i8: + the query expansion).  hm_knn2_resident_runs_exchange: the same with the exchange of
+ * hm_knn2_resident_exchange.  hm_knn2_runs: over packed rows -- the selected rows are gathered into the workspace
+ * (36 bytes per selected row), hm_knn2 runs over them, and one small kernel maps the keys back.
+ * hm_runs_workspace_bytes: workspace of the resident entries (prepared != 0, variant I8 / F4 / AUTO) or of
+ * hm_knn2_runs (prepared == 0, any variant); 0 for invalid runs.  Nothing is sized by unselected rows.
+ * hm_describe_runs_launch: host arithmetic, no device needed -- the resident launch for this selection as text (as
+ * hm_describe_launch) and, when pieces_host != NULL, the tile walk: pieces_host[v] = (split, physical tile, first row,
+ * end row) of virtual tile v, rows clipped to the run.  Returns the number of virtual tiles, or an hm_status < 0. */
+HM_API size_t hm_runs_workspace_bytes(int64_t nq, const int64_t* runs_host, int64_t n_runs, int prepared, int variant);
+HM_API int hm_describe_runs_launch(int64_t nq, int64_t nt, const int64_t* runs_host, int64_t n_runs, int variant,
+                                   char* buf, size_t buf_bytes, int64_t* pieces_host);
+HM_API int hm_knn2_resident_runs(const uint8_t* query, int64_t nq, int64_t q_stride, const void* train_prepared,
+                                 int64_t nt, const int64_t* runs_host, const int64_t* runs_dev, int64_t n_runs,
+                                 uint64_t train_base, uint64_t* out_keys, int variant, void* workspace,
+                                 size_t workspace_bytes, void* stream);
+HM_API int hm_knn2_resident_runs_exchange(const uint8_t* query, int64_t nq, int64_t q_stride, const void* train_prepared,
+                                          int64_t nt, const int64_t* runs_host, const int64_t* runs_dev, int64_t n_runs,
+                                          uint64_t train_base, int world, int rank, void* const* peer_buffers_host,
+                                          int64_t max_rows, uint32_t epoch, uint64_t* out_keys, int variant,
+                                          void* workspace, size_t workspace_bytes, void* stream);
+HM_API int hm_knn2_runs(const uint8_t* query, int64_t nq, int64_t q_stride, const uint8_t* train, int64_t nt,
+                        int64_t t_stride, const int64_t* runs_host, const int64_t* runs_dev, int64_t n_runs,
+                        uint64_t train_base, uint64_t* out_keys, int variant, void* workspace, size_t workspace_bytes,
+                        void* stream);
+
 /* ---- tensor-core operand preparation (resident keyframe database) ---------------------
  * `variant` selects the operand format: HM_VARIANT_I8, HM_VARIANT_F4, or HM_VARIANT_AUTO = the
  * default tensor-core core (hm_default_tensor_variant()).  A prepared image must be consumed with the

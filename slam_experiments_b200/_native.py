@@ -35,6 +35,8 @@ EXPORTS = (
     "hm_describe_launch",
     "hm_knn2", "hm_knn2_batched", "hm_default_tensor_variant", "hm_prepared_bytes", "hm_prepared_workspace_bytes", "hm_prepare", "hm_knn2_prepared", "hm_knn2_prepared_partials", "hm_knn2_prepared_exchange",
     "hm_resident_workspace_bytes", "hm_knn2_resident", "hm_knn2_resident_exchange",
+    "hm_runs_workspace_bytes", "hm_describe_runs_launch", "hm_knn2_resident_runs", "hm_knn2_resident_runs_exchange",
+    "hm_knn2_runs",
     "hm_merge_top2", "hm_exchange_bytes", "hm_exchange_merge", "hm_filter_matches", "hm_match_fused", "hm_gather_points", "hm_rasterize_mask",
     "hm_db_mutual_workspace_bytes", "hm_db_mutual_flags", "hm_db_filter",
     "hm_context_create", "hm_context_destroy", "hm_knn2_host", "hm_match_host", "hm_frame_put", "hm_frame_match",
@@ -85,6 +87,17 @@ def _declare(L):
     L.hm_knn2_resident.argtypes = [vp, i64, i64, vp, i64, u64, vp, ci, vp, sz, vp]
     L.hm_knn2_resident_exchange.restype = ci
     L.hm_knn2_resident_exchange.argtypes = [vp, i64, i64, vp, i64, u64, ci, ci, vp, i64, c.c_uint32, vp, ci, vp, sz, vp]
+    L.hm_runs_workspace_bytes.restype = sz
+    L.hm_runs_workspace_bytes.argtypes = [i64, vp, i64, ci, ci]
+    L.hm_describe_runs_launch.restype = ci
+    L.hm_describe_runs_launch.argtypes = [i64, i64, vp, i64, ci, c.c_char_p, sz, vp]
+    L.hm_knn2_resident_runs.restype = ci
+    L.hm_knn2_resident_runs.argtypes = [vp, i64, i64, vp, i64, vp, vp, i64, u64, vp, ci, vp, sz, vp]
+    L.hm_knn2_resident_runs_exchange.restype = ci
+    L.hm_knn2_resident_runs_exchange.argtypes = [vp, i64, i64, vp, i64, vp, vp, i64, u64, ci, ci, vp, i64, c.c_uint32,
+                                                 vp, ci, vp, sz, vp]
+    L.hm_knn2_runs.restype = ci
+    L.hm_knn2_runs.argtypes = [vp, i64, i64, vp, i64, i64, vp, vp, i64, u64, vp, ci, vp, sz, vp]
     L.hm_merge_top2.restype = ci
     L.hm_merge_top2.argtypes = [vp, ci, i64, vp, vp]
     L.hm_exchange_bytes.restype = sz
@@ -363,6 +376,87 @@ def knn2_resident_exchange(query: torch.Tensor, train_prepared: torch.Tensor, nt
         check(L.hm_knn2_resident_exchange(query.data_ptr(), nq, query.stride(0), train_prepared.data_ptr(), nt, train_base,
                                           world, rank, peer_ptrs, max_rows, epoch, out.data_ptr(), v, ws.data_ptr(),
                                           ws.numel(), _stream_ptr(dev)), "hm_knn2_resident_exchange")
+    return out
+
+
+# ---- selections of train rows as runs (include/hm_matcher.h, "search a selection of the train rows") -------------
+def run_table(runs: np.ndarray) -> np.ndarray:
+    """The device layout of a run list ``int64 [n, 2]`` (lo, hi): ``int64 [n, 4]`` = lo, hi, the 128-row tiles and the
+    rows of the runs before it."""
+    runs = np.ascontiguousarray(runs, dtype=np.int64).reshape(-1, 2)
+    tiles = -(-runs[:, 1] // 128) - runs[:, 0] // 128
+    rows = runs[:, 1] - runs[:, 0]
+    out = np.empty((runs.shape[0], 4), np.int64)
+    out[:, :2] = runs
+    out[:, 2] = np.cumsum(tiles) - tiles
+    out[:, 3] = np.cumsum(rows) - rows
+    return out
+
+
+def runs_workspace_bytes(nq: int, runs: np.ndarray, prepared: bool, variant="auto") -> int:
+    runs = np.ascontiguousarray(runs, dtype=np.int64).reshape(-1, 2)
+    v = tensor_variant(variant) if prepared else variant_id(variant)
+    return int(lib().hm_runs_workspace_bytes(nq, runs.ctypes.data, runs.shape[0], int(prepared), v))
+
+
+def describe_runs_launch(nq: int, nt: int, runs: np.ndarray, variant="auto", pieces: bool = False):
+    """``hm_describe_runs_launch`` (host arithmetic, no device needed): the resident launch of a run list as text, and
+    with ``pieces`` the tile walk ``int64 [T, 4]`` = (split, physical tile, first row, end row) per virtual tile."""
+    runs = np.ascontiguousarray(runs, dtype=np.int64).reshape(-1, 2)
+    L = lib()
+    n = L.hm_describe_runs_launch(nq, nt, runs.ctypes.data, runs.shape[0], tensor_variant(variant), None, 0, None)
+    if n < 0:
+        raise NativeError(f"hm_describe_runs_launch failed with status {n}: {last_error()}")
+    buf = ctypes.create_string_buffer(256)
+    out = np.zeros((n, 4), np.int64)
+    check(min(0, L.hm_describe_runs_launch(nq, nt, runs.ctypes.data, runs.shape[0], tensor_variant(variant), buf, 256,
+                                           out.ctypes.data if pieces and n else None)), "hm_describe_runs_launch")
+    return (buf.value.decode(), out) if pieces else buf.value.decode()
+
+
+def knn2_keys_resident_runs(query: torch.Tensor, train_prepared: torch.Tensor, nt: int, runs: np.ndarray,
+                            runs_dev: torch.Tensor, train_base: int = 0, variant="auto", exchange=None) -> torch.Tensor:
+    """``hm_knn2_resident_runs`` (``exchange`` = (world, rank, peer_ptrs, max_rows, epoch):
+    ``hm_knn2_resident_runs_exchange``): top-2 keys over the runs ``[lo, hi)`` of a resident prepared database.
+    ``runs_dev`` is :func:`run_table` of ``runs`` on the device."""
+    _check_desc(query, "query")
+    dev = query.device
+    nq = query.shape[0]
+    runs = np.ascontiguousarray(runs, dtype=np.int64).reshape(-1, 2)
+    out = torch.empty((nq, 2), dtype=torch.int64, device=dev)
+    v = tensor_variant(variant)
+    L = lib()
+    with on_device(dev):
+        ws = workspace(L.hm_runs_workspace_bytes(nq, runs.ctypes.data, runs.shape[0], 1, v), dev)
+        if exchange is None:
+            check(L.hm_knn2_resident_runs(query.data_ptr(), nq, query.stride(0), train_prepared.data_ptr(), nt,
+                                          runs.ctypes.data, runs_dev.data_ptr(), runs.shape[0], train_base, out.data_ptr(),
+                                          v, ws.data_ptr(), ws.numel(), _stream_ptr(dev)), "hm_knn2_resident_runs")
+        else:
+            world, rank, peer_ptrs, max_rows, epoch = exchange
+            check(L.hm_knn2_resident_runs_exchange(query.data_ptr(), nq, query.stride(0), train_prepared.data_ptr(), nt,
+                                                   runs.ctypes.data, runs_dev.data_ptr(), runs.shape[0], train_base, world,
+                                                   rank, peer_ptrs, max_rows, epoch, out.data_ptr(), v, ws.data_ptr(),
+                                                   ws.numel(), _stream_ptr(dev)), "hm_knn2_resident_runs_exchange")
+    return out
+
+
+def knn2_keys_runs(query: torch.Tensor, train: torch.Tensor, runs: np.ndarray, runs_dev: torch.Tensor,
+                   train_base: int = 0, variant="auto") -> torch.Tensor:
+    """``hm_knn2_runs``: top-2 keys over the runs ``[lo, hi)`` of packed train rows (gathered into the workspace)."""
+    _check_desc(query, "query")
+    _check_desc(train, "train")
+    dev = query.device
+    nq, nt = query.shape[0], train.shape[0]
+    runs = np.ascontiguousarray(runs, dtype=np.int64).reshape(-1, 2)
+    out = torch.empty((nq, 2), dtype=torch.int64, device=dev)
+    v = variant_id(variant)
+    L = lib()
+    with on_device(dev):
+        ws = workspace(L.hm_runs_workspace_bytes(nq, runs.ctypes.data, runs.shape[0], 0, v), dev)
+        check(L.hm_knn2_runs(query.data_ptr(), nq, query.stride(0) if nq else DESC_BYTES, train.data_ptr(), nt,
+                             train.stride(0) if nt else DESC_BYTES, runs.ctypes.data, runs_dev.data_ptr(), runs.shape[0],
+                             train_base, out.data_ptr(), v, ws.data_ptr(), ws.numel(), _stream_ptr(dev)), "hm_knn2_runs")
     return out
 
 

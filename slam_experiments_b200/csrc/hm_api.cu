@@ -8,6 +8,7 @@
 
 #include <mutex>
 #include <new>
+#include <vector>
 
 #include "hm_common.cuh"
 
@@ -178,6 +179,87 @@ int knn2_dispatch(const KnnProblem& p, unsigned long long* out, int variant, voi
         case HM_VARIANT_F4: return launch_tc_knn2(p, out, ws, ws_bytes, di.sm_count, v, stream);
         default: set_error("unknown variant %d", variant); return HM_ERR_INVALID_ARGUMENT;
     }
+}
+
+
+// ---- selections of train rows as runs (hm_knn2_resident_runs, hm_knn2_runs) ----------------------------------------
+// runs_host[n_runs][2] must be non-empty, ascending and disjoint within [0, nt), nt < 2^32 (32-bit trainIdx).  On
+// success *tot holds the 128-row tiles the runs touch and the rows they hold; with `four` also the kRunFields layout of
+// the device array (the host's own copy, for the planner's walk).
+int check_runs(const int64_t* runs, long long n_runs, long long nt, RunTotals* tot, std::vector<long long>* four)
+{
+    if (n_runs < 0 || n_runs > 0x7FFFFFFFll || (n_runs > 0 && !runs)) {
+        set_error("runs: bad count %lld or null host array", n_runs);
+        return HM_ERR_INVALID_ARGUMENT;
+    }
+    if (nt < 0 || nt >= (1ll << 32)) {
+        set_error("runs: train rows %lld outside [0, 2^32)", nt);
+        return HM_ERR_INVALID_ARGUMENT;
+    }
+    long long prev = 0, tiles = 0, rows = 0;
+    if (four) four->clear();
+    for (long long i = 0; i < n_runs; ++i) {
+        const long long lo = runs[2 * i], hi = runs[2 * i + 1];
+        if (lo < prev || hi <= lo || hi > nt) {
+            set_error("run %lld = [%lld, %lld): runs must be non-empty, ascending and disjoint within [0, %lld)", i, lo, hi,
+                      nt);
+            return HM_ERR_INVALID_ARGUMENT;
+        }
+        if (four) four->insert(four->end(), {lo, hi, tiles, rows});
+        tiles += ceil_div(hi, 128) - lo / 128;
+        rows += hi - lo;
+        prev = hi;
+    }
+    if (tiles > 0x7FFFFFFFll) {
+        set_error("runs: %lld tiles to walk", tiles);
+        return HM_ERR_UNSUPPORTED;
+    }
+    tot->tiles = tiles;
+    tot->rows = rows;
+    return HM_OK;
+}
+
+int check_runs_dev(const int64_t* runs_dev, long long n_runs)
+{
+    if (n_runs > 0 && (!runs_dev || (reinterpret_cast<uintptr_t>(runs_dev) & 7))) {
+        set_error("runs_dev: null or not 8-byte aligned");
+        return HM_ERR_INVALID_ARGUMENT;
+    }
+    return HM_OK;
+}
+
+// hm_knn2_runs: [map: rows x u32 | gathered rows: rows x 32 B | workspace of hm_knn2 over the gathered rows]
+size_t packed_runs_workspace(long long nq, long long rows, int variant, int sm_count)
+{
+    return align_up((size_t)rows * 4) + align_up((size_t)rows * HM_DESC_BYTES) + knn_workspace(nq, rows, 1, variant, sm_count);
+}
+
+// selected row j -> gathered[j] and map[j] = its shard-local row; one thread per 16 bytes.  The map ascends with j, so
+// the stable order of the gathered problem is the stable order of the rows.
+__global__ void hm_runs_gather_kernel(const uint8_t* train, long long t_stride, const long long* runs, int n_runs,
+                                      long long rows, uint8_t* gathered, unsigned* map)
+{
+    const long long o = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (o >= rows * 2) return;
+    const long long j = o >> 1;
+    int a = 0, b = n_runs - 1;                         // the last run whose row prefix is <= j
+    while (a < b) {
+        const int m = (a + b + 1) >> 1;
+        if (runs[kRunFields * m + 3] <= j) a = m;
+        else b = m - 1;
+    }
+    const long long row = runs[kRunFields * a] + (j - runs[kRunFields * a + 3]);
+    reinterpret_cast<uint4*>(gathered)[o] = *reinterpret_cast<const uint4*>(train + row * t_stride + (o & 1) * 16);
+    if (!(o & 1)) map[j] = (unsigned)row;
+}
+
+__global__ void hm_runs_remap_kernel(unsigned long long* keys, long long n, const unsigned* map,
+                                     unsigned long long train_base)
+{
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const unsigned long long k = keys[i];
+    if (k != kNoMatch) keys[i] = (k & 0xFFFFFFFF00000000ull) + train_base + map[k & 0xFFFFFFFFull];
 }
 
 }  // namespace
@@ -434,6 +516,170 @@ HM_API int hm_knn2_resident_exchange(const uint8_t* query, int64_t nq, int64_t q
     if ((rc = fill_exchange_args(&x, world, rank, peer_buffers_host, max_rows, epoch, nq)) != HM_OK) return rc;
     return knn2_resident_common(query, nq, q_stride, train_prepared, nt, train_base, out_keys, variant, workspace,
                                 workspace_bytes, stream, &x, "hm_knn2_resident_exchange");
+}
+
+HM_API size_t hm_runs_workspace_bytes(int64_t nq, const int64_t* runs_host, int64_t n_runs, int prepared, int variant)
+{
+    DeviceInfo di;
+    int sm = 148;
+    if (device_info(&di) == HM_OK) sm = di.sm_count;
+    RunTotals tot;
+    if (nq < 0 || check_runs(runs_host, n_runs, (1ll << 32) - 1, &tot, nullptr) != HM_OK) return 0;
+    if (prepared) {
+        const int v = resolve_tensor_variant(variant);
+        if (v < 0) return 0;
+        if (nq == 0 || tot.tiles == 0) return 256;
+        return align_up(tc_resident_workspace_bytes(nq, tot.tiles * 128, sm, v));
+    }
+    if (variant < HM_VARIANT_AUTO || variant > HM_VARIANT_F4) return 0;
+    if (nq == 0 || tot.rows == 0) return 256;
+    return align_up(packed_runs_workspace(nq, tot.rows, variant, sm));
+}
+
+HM_API int hm_describe_runs_launch(int64_t nq, int64_t nt, const int64_t* runs_host, int64_t n_runs, int variant,
+                                   char* buf, size_t buf_bytes, int64_t* pieces_host)
+{
+    if (nq <= 0) {
+        set_error("hm_describe_runs_launch: needs query rows");
+        return HM_ERR_INVALID_ARGUMENT;
+    }
+    const int v = resolve_tensor_variant(variant);
+    if (v < 0) return v;
+    RunTotals tot;
+    std::vector<long long> four;
+    const int rc = check_runs(runs_host, n_runs, nt, &tot, &four);
+    if (rc != HM_OK) return rc;
+    if (n_runs == 0) {
+        if (buf && buf_bytes) snprintf(buf, buf_bytes, "no launch: empty selection");
+        return 0;
+    }
+    DeviceInfo di;
+    int sm = 148;   // B200; the real count when a device is visible
+    if (device_info(&di) == HM_OK) sm = di.sm_count;
+    describe_tc_runs(nq, four.data(), (int)n_runs, tot.tiles, sm, v, buf, buf_bytes,
+                     reinterpret_cast<long long*>(pieces_host));
+    return (int)tot.tiles;
+}
+
+static int knn2_resident_runs_common(const uint8_t* query, int64_t nq, int64_t q_stride, const void* train_prepared,
+                                     int64_t nt, const int64_t* runs_host, const int64_t* runs_dev, int64_t n_runs,
+                                     uint64_t train_base, uint64_t* out_keys, int variant, void* workspace,
+                                     size_t workspace_bytes, void* stream, const ExchangeArgs* x, const char* who)
+{
+    DeviceInfo di;
+    int rc = device_info(&di);
+    if (rc != HM_OK) return rc;
+    const int v = resolve_tensor_variant(variant);
+    if (v < 0) return v;
+    RunTotals tot;
+    if ((rc = check_runs(runs_host, n_runs, nt, &tot, nullptr)) != HM_OK) return rc;
+    if ((rc = check_runs_dev(runs_dev, n_runs)) != HM_OK) return rc;
+    if (nq < 0) {
+        set_error("%s: negative row count", who);
+        return HM_ERR_INVALID_ARGUMENT;
+    }
+    if (nq == 0) return HM_OK;
+    if (!out_keys) {
+        set_error("%s: out_keys is null", who);
+        return HM_ERR_INVALID_ARGUMENT;
+    }
+    if ((rc = check_rows(query, nq, q_stride, "query")) != HM_OK) return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (n_runs == 0) {
+        if (x) {
+            set_error("%s: needs at least one run (a rank without selected rows joins through hm_exchange_merge)", who);
+            return HM_ERR_INVALID_ARGUMENT;
+        }
+        return fill_no_match(reinterpret_cast<unsigned long long*>(out_keys), nq * 2, st);
+    }
+    if (!train_prepared || (reinterpret_cast<uintptr_t>(train_prepared) & 15)) {
+        set_error("%s: the prepared database must be non-null and 16-byte aligned", who);
+        return HM_ERR_INVALID_ARGUMENT;
+    }
+    const RunArgs ra{reinterpret_cast<const long long*>(runs_dev), (int)n_runs};
+    return launch_tc_knn2_resident_runs(query, nq, q_stride, train_prepared, nt, ra, tot, train_base,
+                                        reinterpret_cast<unsigned long long*>(out_keys), workspace, workspace_bytes,
+                                        di.sm_count, v, st, x);
+}
+
+HM_API int hm_knn2_resident_runs(const uint8_t* query, int64_t nq, int64_t q_stride, const void* train_prepared,
+                                 int64_t nt, const int64_t* runs_host, const int64_t* runs_dev, int64_t n_runs,
+                                 uint64_t train_base, uint64_t* out_keys, int variant, void* workspace,
+                                 size_t workspace_bytes, void* stream)
+{
+    return knn2_resident_runs_common(query, nq, q_stride, train_prepared, nt, runs_host, runs_dev, n_runs, train_base,
+                                     out_keys, variant, workspace, workspace_bytes, stream, nullptr,
+                                     "hm_knn2_resident_runs");
+}
+
+HM_API int hm_knn2_resident_runs_exchange(const uint8_t* query, int64_t nq, int64_t q_stride, const void* train_prepared,
+                                          int64_t nt, const int64_t* runs_host, const int64_t* runs_dev, int64_t n_runs,
+                                          uint64_t train_base, int world, int rank, void* const* peer_buffers_host,
+                                          int64_t max_rows, uint32_t epoch, uint64_t* out_keys, int variant,
+                                          void* workspace, size_t workspace_bytes, void* stream)
+{
+    ExchangeArgs x;
+    DeviceInfo di;
+    int rc = device_info(&di);
+    if (rc != HM_OK) return rc;
+    if (nq <= 0) {
+        set_error("hm_knn2_resident_runs_exchange: needs query rows (every rank posts its flags)");
+        return HM_ERR_INVALID_ARGUMENT;
+    }
+    if ((rc = fill_exchange_args(&x, world, rank, peer_buffers_host, max_rows, epoch, nq)) != HM_OK) return rc;
+    return knn2_resident_runs_common(query, nq, q_stride, train_prepared, nt, runs_host, runs_dev, n_runs, train_base,
+                                     out_keys, variant, workspace, workspace_bytes, stream, &x,
+                                     "hm_knn2_resident_runs_exchange");
+}
+
+HM_API int hm_knn2_runs(const uint8_t* query, int64_t nq, int64_t q_stride, const uint8_t* train, int64_t nt,
+                        int64_t t_stride, const int64_t* runs_host, const int64_t* runs_dev, int64_t n_runs,
+                        uint64_t train_base, uint64_t* out_keys, int variant, void* workspace, size_t workspace_bytes,
+                        void* stream)
+{
+    DeviceInfo di;
+    int rc = device_info(&di);
+    if (rc != HM_OK) return rc;
+    if (variant < HM_VARIANT_AUTO || variant > HM_VARIANT_F4) {
+        set_error("unknown variant %d", variant);
+        return HM_ERR_INVALID_ARGUMENT;
+    }
+    RunTotals tot;
+    if ((rc = check_runs(runs_host, n_runs, nt, &tot, nullptr)) != HM_OK) return rc;
+    if ((rc = check_runs_dev(runs_dev, n_runs)) != HM_OK) return rc;
+    if (nq < 0) {
+        set_error("hm_knn2_runs: negative row count");
+        return HM_ERR_INVALID_ARGUMENT;
+    }
+    if (nq == 0) return HM_OK;
+    if (!out_keys) {
+        set_error("hm_knn2_runs: out_keys is null");
+        return HM_ERR_INVALID_ARGUMENT;
+    }
+    if ((rc = check_rows(query, nq, q_stride, "query")) != HM_OK) return rc;
+    if ((rc = check_rows(train, nt, t_stride, "train")) != HM_OK) return rc;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    unsigned long long* out = reinterpret_cast<unsigned long long*>(out_keys);
+    if (tot.rows == 0) return fill_no_match(out, nq * 2, st);
+    const size_t need = packed_runs_workspace(nq, tot.rows, variant, di.sm_count);
+    if (!workspace || workspace_bytes < need) {
+        set_error("workspace too small: need %zu bytes, got %zu", need, workspace_bytes);
+        return HM_ERR_WORKSPACE;
+    }
+    unsigned* map = static_cast<unsigned*>(workspace);
+    uint8_t* gathered = static_cast<uint8_t*>(workspace) + align_up((size_t)tot.rows * 4);
+    const size_t head = align_up((size_t)tot.rows * 4) + align_up((size_t)tot.rows * HM_DESC_BYTES);
+    hm_runs_gather_kernel<<<(unsigned)ceil_div(tot.rows * 2, 256), 256, 0, st>>>(
+        train, t_stride, reinterpret_cast<const long long*>(runs_dev), (int)n_runs, tot.rows, gathered, map);
+    HM_CUDA_CHECK(cudaGetLastError());
+    KnnProblem p{};
+    p.q = query; p.t = gathered; p.nq = nq; p.nt = tot.rows; p.q_stride = q_stride; p.t_stride = HM_DESC_BYTES;
+    p.batch = 1; p.train_base = 0;
+    if ((rc = knn2_dispatch(p, out, variant, static_cast<uint8_t*>(workspace) + head, workspace_bytes - head, st)) != HM_OK)
+        return rc;
+    hm_runs_remap_kernel<<<(unsigned)ceil_div(nq * 2, 256), 256, 0, st>>>(out, nq * 2, map, train_base);
+    HM_CUDA_CHECK(cudaGetLastError());
+    return HM_OK;
 }
 
 HM_API int hm_merge_top2(const uint64_t* keys, int groups, int64_t rows, uint64_t* out_keys, void* stream)

@@ -51,6 +51,19 @@ struct RatioLut {
     unsigned short v[257];
 };
 
+// A selection of train rows as ascending, disjoint, non-empty runs [lo, hi) of rows (hm_knn2_resident_runs,
+// hm_knn2_runs).  The device array holds kRunFields int64 per run: lo, hi, the tiles of 128 rows the runs before it
+// touch (their sum of ceil(hi / 128) - floor(lo / 128)) and the rows the runs before it hold.
+constexpr int kRunFields = 4;
+struct RunArgs {
+    const long long* runs;        // device [n_runs][kRunFields]
+    int n_runs;
+};
+// checked on the host from the caller's [n_runs][2] copy: tiles / rows of the whole selection
+struct RunTotals {
+    long long tiles, rows;
+};
+
 // Ratio test + candidate selection on a row's final keys, run by the k-NN kernel that produced them (row P of
 // SURVEY.md 8a: /root/reference/feature_matchers.py:34,39 extended by Lowe's test and the mutual check).  A row that
 // passes the ratio test marks its best train row as a CANDIDATE column; the swapped pass of the mutual check then
@@ -255,6 +268,16 @@ int launch_tc_knn2_resident(const uint8_t* qbits, long long nq, long long q_stri
                             int sm_count, int variant, cudaStream_t stream, const ExchangeArgs* exchange = nullptr);
 int fill_exchange_args(ExchangeArgs* x, int world, int rank, void* const* peers, long long max_rows, unsigned epoch,
                        long long rows);
+// the same over the selected runs of the prepared rows only; `totals` from the host copy of the runs (workspace:
+// tc_resident_workspace_bytes(nq, totals.tiles * 128, ...))
+int launch_tc_knn2_resident_runs(const uint8_t* qbits, long long nq, long long q_stride, const void* tprep, long long nt,
+                                 const RunArgs& runs, const RunTotals& totals, unsigned long long train_base,
+                                 unsigned long long* out, void* ws, size_t ws_bytes, int sm_count, int variant,
+                                 cudaStream_t stream, const ExchangeArgs* exchange = nullptr);
+// the physical tile sequence the CTAs of a run launch walk: out[v] = (split, tile, first column, end column) for
+// virtual tile v, columns shard-local and clipped to the run (host arithmetic, the kernel's own walk)
+void describe_tc_runs(long long nq, const long long* runs_host4, int n_runs, long long tiles, int sm_count, int variant,
+                      char* buf, size_t n, long long* pieces);
 size_t tc_workspace_bytes(long long nq, long long nt, int batch, int sm_count, bool with_prepare, int variant);
 int launch_tc_knn2(const KnnProblem& p, unsigned long long* out, void* ws, size_t ws_bytes, int sm_count,
                    int variant, cudaStream_t stream);

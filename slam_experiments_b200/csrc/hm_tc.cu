@@ -164,6 +164,44 @@ constexpr int kScaleCols = 32;
 constexpr int kScaleCol = kTmemCols - kScaleCols;
 static_assert(CoreF4::kUnits * CoreF4::kTileN <= kScaleCol, "accumulator units must end before the scale factors");
 
+// ---- run walk (hm_knn2_resident_runs) ------------------------------------------------------------
+// A selection of rows is a list of ascending, disjoint runs [lo, hi) (RunArgs).  Its virtual tiles [0, T) are the
+// 128-row tiles each run touches, run after run: a tile two runs share (across a short unselected stretch) appears
+// once per run, the lower run first.  Split s of a launch takes virtual tiles [s * tiles_per_split, ...).  The kernel's
+// producer and epilogue warps and describe_tc_runs walk the same sequence with this cursor.
+struct RunCursor {
+    int r;                       // current run
+    int tile, end;               // physical tile; one past the run's last tile
+    unsigned lo, hi;             // the run's rows (shard-local): columns outside [lo, hi) must never win
+    __host__ __device__ __forceinline__ void load(const long long* runs, int rr)
+    {
+        r = rr;
+        const long long a = runs[kRunFields * rr], b = runs[kRunFields * rr + 1];
+        lo = (unsigned)a;
+        hi = (unsigned)b;
+        tile = (int)(a / kRowBlock);
+        end = (int)((b + kRowBlock - 1) / kRowBlock);
+    }
+    // position at virtual tile v: the last run whose tile prefix is <= v (prefixes strictly increase: runs are non-empty)
+    __host__ __device__ __forceinline__ void seek(const long long* runs, int n_runs, long long v)
+    {
+        int a = 0, b = n_runs - 1;
+        while (a < b) {
+            const int m = (a + b + 1) >> 1;
+            if (runs[kRunFields * m + 2] <= v) a = m;
+            else b = m - 1;
+        }
+        load(runs, a);
+        tile += (int)(v - runs[kRunFields * a + 2]);
+    }
+    // the next virtual tile; only called when there is one
+    __host__ __device__ __forceinline__ void next(const long long* runs)
+    {
+        if (++tile == end) load(runs, r + 1);
+    }
+};
+static_assert(CoreI8::kTileN == kRowBlock && CoreF4::kTileN == kRowBlock, "the run walk counts tiles of kRowBlock rows");
+
 // ------------------------------------------------------------------------------------------
 // hm_prepare: packed bits -> +/-1 in the tiled swizzled layout.  One thread writes one 16-byte
 // chunk (16 descriptor bits as int8, 32 as e2m1); consecutive threads write consecutive chunks.
@@ -406,6 +444,15 @@ __device__ __forceinline__ void mask_tail(uint32_t* r, unsigned colbase, unsigne
     }
 }
 
+// run walk: columns outside the current run [lo, hi) -- in the run's first and last tile only -- must never win
+template <class C, int kN>
+__device__ __forceinline__ void mask_outside(uint32_t* r, unsigned colbase, unsigned lo, unsigned hi)
+{
+#pragma unroll
+    for (int j = 0; j < kN; ++j)
+        if (colbase + j < lo || colbase + j >= hi) r[j] = C::kLowestBits;
+}
+
 // the shared row thresholds are refreshed on each of a CTA's first kFloorDenseTiles tiles, then on every 16th
 constexpr int kFloorDenseTiles = 32;
 constexpr int kFloorLateMask = 15;
@@ -428,8 +475,10 @@ __device__ __forceinline__ void issue_half(int h, uint32_t a_block, uint32_t b_s
     }
 }
 
-template <class C, int kMode>
-__device__ __forceinline__ void tc_knn2_body(const TcParams& P)
+// kRuns: the train tiles come from the run list R (RunCursor) instead of tile_begin + i; columns are physical
+// (shard-local rows, first_row = 0), so the final fold needs no remapping
+template <class C, int kMode, bool kRuns = false>
+__device__ __forceinline__ void tc_knn2_body(const TcParams& P, const RunArgs& R = RunArgs{})
 {
     constexpr bool kFloor = kMode == 1;
     using Acc = typename C::Acc;
@@ -567,13 +616,20 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
             }
             const uint8_t* tsrc = P.tprep + (long long)b * P.t_padded * C::kRowBytes;
             const uint32_t piece = kBStageBytes / cs;     // this CTA fetches 1/cs of every tile and multicasts it
+            RunCursor cur;
+            if constexpr (kRuns) cur.seek(R.runs, R.n_runs, tile_begin);
             for (int i = 0; i < my_tiles; ++i) {
                 const int stage = i % kStages;
                 const uint32_t use = i / kStages;
                 bounded_wait(&empty_bar[stage], (use & 1) ^ 1, P.error_flag);
                 ptx::mbar_arrive_expect_tx(&full_bar[stage], kBStageBytes);
                 uint8_t* dst = smem_b + stage * kBStageBytes + crank * piece;
-                const uint8_t* src = tsrc + (long long)(tile_begin + i) * kBStageBytes + crank * piece;
+                int tile = tile_begin + i;
+                if constexpr (kRuns) {
+                    tile = cur.tile;
+                    if (i + 1 < my_tiles) cur.next(R.runs);
+                }
+                const uint8_t* src = tsrc + (long long)tile * kBStageBytes + crank * piece;
                 if (cs > 1) ptx::bulk_g2s_multicast(dst, src, piece, &full_bar[stage], cmask);
                 else        ptx::bulk_g2s(dst, src, piece, &full_bar[stage]);
             }
@@ -675,8 +731,10 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
         for (int e = 0; e < 4; ++e) s.sa[e] = s.sb[e] = 0;
         s.f = C::floor_from(0);                           // below every possible dot
         unsigned floor_code = 0;                          // largest threshold code read or published so far
-        const long long first_row = (long long)tile_begin * kTileN;
+        const long long first_row = kRuns ? 0ll : (long long)tile_begin * kTileN;
         const unsigned limit = (unsigned)min((long long)my_tiles * kTileN, P.nt - first_row);
+        RunCursor cur;
+        if constexpr (kRuns) cur.seek(R.runs, R.n_runs, tile_begin);
         // barrier addresses of the tile loop, derived from an opaque copy of the shared-memory base
         const uint32_t bars_addr = ptx::lds_volatile_u32(ptx::smem_u32(smem_base_slot)) + kABytes + kStages * kBStageBytes;
         const uint32_t unit_full_addr = bars_addr + (2 * kStages + 1) * 8;
@@ -709,7 +767,13 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
             bounded_wait_addr(unit_full_addr + unit * 8, unit_use & 1, P.error_flag);
             ptx::tc_fence_after();
             const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + unit * kTileN + half * kCols;
-            const unsigned colbase = (unsigned)i * kTileN + half * kCols;
+            unsigned colbase = (unsigned)i * kTileN + half * kCols;
+            bool run_edge = false;
+            if constexpr (kRuns) {
+                colbase = (unsigned)cur.tile * kTileN + half * kCols;
+                // one uniform compare per tile; only a run's partial first and last tiles take the masking branch
+                run_edge = colbase < cur.lo || colbase + kCols > cur.hi;
+            }
             if constexpr (C::kColSplit == 1) {
                 // all four 32-column loads are issued before the first scan so their latencies overlap
                 uint32_t r0[32], r1[32], r2[32], r3[32];
@@ -723,7 +787,14 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
                 ptx::tc_fence_before();
                 __syncwarp();
                 if (ptx::elect_one()) ptx::mbar_arrive_addr(unit_empty_addr + unit * 8);
-                if (colbase + kCols > limit) {            // last tile of the train set only
+                if constexpr (kRuns) {
+                    if (run_edge) {
+                        mask_outside<C, 32>(r0, colbase, cur.lo, cur.hi);
+                        mask_outside<C, 32>(r1, colbase + 32, cur.lo, cur.hi);
+                        mask_outside<C, 32>(r2, colbase + 64, cur.lo, cur.hi);
+                        mask_outside<C, 32>(r3, colbase + 96, cur.lo, cur.hi);
+                    }
+                } else if (colbase + kCols > limit) {     // last tile of the train set only
                     mask_tail<C, 32>(r0, colbase, limit);
                     mask_tail<C, 32>(r1, colbase + 32, limit);
                     mask_tail<C, 32>(r2, colbase + 64, limit);
@@ -746,11 +817,18 @@ __device__ __forceinline__ void tc_knn2_body(const TcParams& P)
                 // software pipelining over half items -- two 32-register buffers, the next item's first half loaded
                 // while this item's second half is scanned -- 882.  The flat 64-column tree below measured 867 then;
                 // with the group-level scan it measured a wash and was adopted, DESIGN.md §3.3 items 10-11.)
-                mask_tail<C, 64>(r, colbase, limit);
+                if constexpr (kRuns) {
+                    if (run_edge) mask_outside<C, 64>(r, colbase, cur.lo, cur.hi);
+                } else {
+                    mask_tail<C, 64>(r, colbase, limit);
+                }
                 scan_chunk<C, kMode, 8>(r, colbase, s);          // one compare + branch per 64 columns
             }
             unit += 2;
             if (unit >= kUnits) { unit -= kUnits; ++unit_use; }
+            if constexpr (kRuns) {
+                if (i + 1 < my_tiles) cur.next(R.runs);
+            }
         };
 #pragma unroll 1
         for (int i = 0; i < my_tiles; ++i) process_tile(i);
@@ -850,10 +928,21 @@ __global__ void __launch_bounds__(threads<CoreF4>(), 1) hm_f4_knn2_floor_kernel(
 __global__ void __launch_bounds__(threads<CoreI8>(), 1) hm_i8_knn1_kernel(const TcParams P) { tc_knn2_body<CoreI8, 2>(P); }
 __global__ void __launch_bounds__(threads<CoreF4>(), 1) hm_f4_knn1_kernel(const TcParams P) { tc_knn2_body<CoreF4, 2>(P); }
 
+// top-2 over the selected runs of a resident shard (hm_knn2_resident_runs*): the same bodies walking RunArgs; the floor
+// kernels for split launches, the plain ones for unsplit shapes, the fused exchange through TcParams::xch as above
+__global__ void __launch_bounds__(threads<CoreI8>(), 1) hm_i8_knn2_runs_kernel(const TcParams P, const RunArgs R) { tc_knn2_body<CoreI8, 0, true>(P, R); }
+__global__ void __launch_bounds__(threads<CoreF4>(), 1) hm_f4_knn2_runs_kernel(const TcParams P, const RunArgs R) { tc_knn2_body<CoreF4, 0, true>(P, R); }
+__global__ void __launch_bounds__(threads<CoreI8>(), 1) hm_i8_knn2_runs_floor_kernel(const TcParams P, const RunArgs R) { tc_knn2_body<CoreI8, 1, true>(P, R); }
+__global__ void __launch_bounds__(threads<CoreF4>(), 1) hm_f4_knn2_runs_floor_kernel(const TcParams P, const RunArgs R) { tc_knn2_body<CoreF4, 1, true>(P, R); }
+
 using KernelFn = void (*)(const TcParams);
 template <class C> KernelFn kernel_of(int mode = 0);
 template <> KernelFn kernel_of<CoreI8>(int mode) { return mode == 1 ? hm_i8_knn2_floor_kernel : mode == 2 ? hm_i8_knn1_kernel : hm_i8_knn2_kernel; }
 template <> KernelFn kernel_of<CoreF4>(int mode) { return mode == 1 ? hm_f4_knn2_floor_kernel : mode == 2 ? hm_f4_knn1_kernel : hm_f4_knn2_kernel; }
+using RunsKernelFn = void (*)(const TcParams, const RunArgs);
+template <class C> RunsKernelFn runs_kernel_of(bool floor);
+template <> RunsKernelFn runs_kernel_of<CoreI8>(bool floor) { return floor ? hm_i8_knn2_runs_floor_kernel : hm_i8_knn2_runs_kernel; }
+template <> RunsKernelFn runs_kernel_of<CoreF4>(bool floor) { return floor ? hm_f4_knn2_runs_floor_kernel : hm_f4_knn2_runs_kernel; }
 
 struct TcPlan {
     int ntiles, splits, tiles_per_split;
@@ -896,6 +985,10 @@ cudaError_t ensure_smem_opt_in()
     if (dev >= 0 && done[dev]) return cudaSuccess;
     for (int mode = 0; mode < 3; ++mode) {
         const cudaError_t e = cudaFuncSetAttribute(kernel_of<C>(mode), cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes<C>());
+        if (e != cudaSuccess) return e;
+    }
+    for (int floor = 0; floor < 2; ++floor) {
+        const cudaError_t e = cudaFuncSetAttribute(runs_kernel_of<C>(floor != 0), cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes<C>());
         if (e != cudaSuccess) return e;
     }
     if (dev >= 0) done[dev] = true;
@@ -1016,17 +1109,23 @@ int launch_prepared(const void* qprep, long long nq, const void* tprep, long lon
                     unsigned long long train_base, unsigned long long* out, void* ws, size_t ws_bytes,
                     int sm_count, cudaStream_t stream, const unsigned long long** out_partials,
                     int* out_groups, const ExchangeArgs* exchange, bool top1 = false, const QueryBits* qbits = nullptr,
-                    const SelectArgs* select = nullptr)
+                    const SelectArgs* select = nullptr, const RunArgs* runs = nullptr, long long run_tiles = 0)
 {
     HM_CUDA_CHECK(ensure_smem_opt_in<C>());
-    const TcPlan pl = plan_tc<C>(nq, nt, batch, sm_count);
-    if ((long long)pl.ntiles * C::kTileN > (1ll << 32)) {
+    // a run walk is planned over its virtual tiles exactly as a whole train set over its tiles
+    const long long plan_nt = runs ? run_tiles * C::kTileN : nt;
+    const TcPlan pl = plan_tc<C>(nq, plan_nt, batch, sm_count);
+    if (ceil_div(nt, C::kTileN) * C::kTileN > (1ll << 32)) {
         set_error("train set too large for 32-bit trainIdx");
         return HM_ERR_UNSUPPORTED;
     }
+    if (runs && (batch != 1 || top1 || (qbits && qbits->index) || (select && select->slot_of) || out == nullptr)) {
+        set_error("a run walk is a single top-2 problem with an output buffer");
+        return HM_ERR_INVALID_ARGUMENT;
+    }
     const bool keep_partials = out == nullptr;
     const size_t cbytes = zeroed_bytes(pl.qblocks * batch, nq * batch);
-    const size_t need = 256 + cbytes + partials_bytes<C>(nq, nt, batch, sm_count);
+    const size_t need = 256 + cbytes + partials_bytes<C>(nq, plan_nt, batch, sm_count);
     if (!ws || ws_bytes < need) {
         set_error("workspace too small: need %zu bytes, got %zu", need, ws_bytes);
         return HM_ERR_WORKSPACE;
@@ -1053,7 +1152,7 @@ int launch_prepared(const void* qprep, long long nq, const void* tprep, long lon
     P.q_padded = padded_rows<C>(nq);
     P.t_padded = padded_rows<C>(nt);
     P.tiles_per_split = pl.tiles_per_split;
-    P.ntiles = pl.ntiles;
+    P.ntiles = pl.ntiles;            // run walk: the virtual tiles
     P.train_base = train_base;
     P.error_flag = static_cast<int*>(ws);
     P.clock_probe = reinterpret_cast<long long*>(static_cast<uint8_t*>(ws) + HM_WS_CLOCK_PROBE_OFFSET);   // inside the 256-byte header
@@ -1111,7 +1210,8 @@ int launch_prepared(const void* qprep, long long nq, const void* tprep, long lon
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     profile_mark(true, stream);
-    cudaError_t le = cudaLaunchKernelEx(&cfg, kernel_of<C>(P.row_floor ? 1 : top1 ? 2 : 0), P);
+    cudaError_t le = runs ? cudaLaunchKernelEx(&cfg, runs_kernel_of<C>(P.row_floor != nullptr), P, *runs)
+                          : cudaLaunchKernelEx(&cfg, kernel_of<C>(P.row_floor ? 1 : top1 ? 2 : 0), P);
     profile_mark(false, stream);
     if (le != cudaSuccess) {
         set_error("cudaLaunchKernelEx(tensor-core k-NN kernel, cluster %d) failed: %s", pl.cluster, cudaGetErrorString(le));
@@ -1213,11 +1313,14 @@ size_t tc_resident_workspace_bytes(long long nq, long long nt, int sm_count, int
     return b;
 }
 
-int launch_tc_knn2_resident(const uint8_t* qbits, long long nq, long long q_stride, const void* tprep, long long nt,
-                            unsigned long long train_base, unsigned long long* out, void* ws, size_t ws_bytes,
-                            int sm_count, int variant, cudaStream_t stream, const ExchangeArgs* exchange)
+// runs != nullptr: the walk over the selected runs, planned and sized over run_tiles tiles instead of nt rows
+static int resident_of(const uint8_t* qbits, long long nq, long long q_stride, const void* tprep, long long nt,
+                       unsigned long long train_base, unsigned long long* out, void* ws, size_t ws_bytes, int sm_count,
+                       int variant, cudaStream_t stream, const ExchangeArgs* exchange, const RunArgs* runs,
+                       long long run_tiles)
 {
-    const size_t need = tc_resident_workspace_bytes(nq, nt, sm_count, variant);
+    const long long plan_nt = runs ? run_tiles * kRowBlock : nt;
+    const size_t need = tc_resident_workspace_bytes(nq, plan_nt, sm_count, variant);
     if (!ws || ws_bytes < need) {
         set_error("workspace too small: need %zu bytes, got %zu", need, ws_bytes);
         return HM_ERR_WORKSPACE;
@@ -1225,14 +1328,31 @@ int launch_tc_knn2_resident(const uint8_t* qbits, long long nq, long long q_stri
     if (variant == HM_VARIANT_F4) {
         QueryBits qb{qbits, q_stride, 0};
         return launch_prepared<CoreF4>(nullptr, nq, tprep, nt, 1, train_base, out, ws, ws_bytes, sm_count, stream, nullptr,
-                                       nullptr, exchange, false, &qb);
+                                       nullptr, exchange, false, &qb, nullptr, runs, run_tiles);
     }
-    const size_t head = (tc_workspace_bytes(nq, nt, 1, sm_count, false, variant) + 1023) & ~(size_t)1023;
+    const size_t head = (tc_workspace_bytes(nq, plan_nt, 1, sm_count, false, variant) + 1023) & ~(size_t)1023;
     uint8_t* qprep = static_cast<uint8_t*>(ws) + head;
     const int rc = launch_prepare_of<CoreI8>(qbits, nq, q_stride, 0, 1, qprep, stream);
     if (rc != HM_OK) return rc;
     return launch_prepared<CoreI8>(qprep, nq, tprep, nt, 1, train_base, out, ws, head, sm_count, stream, nullptr, nullptr,
-                                   exchange);
+                                   exchange, false, nullptr, nullptr, runs, run_tiles);
+}
+
+int launch_tc_knn2_resident(const uint8_t* qbits, long long nq, long long q_stride, const void* tprep, long long nt,
+                            unsigned long long train_base, unsigned long long* out, void* ws, size_t ws_bytes,
+                            int sm_count, int variant, cudaStream_t stream, const ExchangeArgs* exchange)
+{
+    return resident_of(qbits, nq, q_stride, tprep, nt, train_base, out, ws, ws_bytes, sm_count, variant, stream, exchange,
+                       nullptr, 0);
+}
+
+int launch_tc_knn2_resident_runs(const uint8_t* qbits, long long nq, long long q_stride, const void* tprep, long long nt,
+                                 const RunArgs& runs, const RunTotals& totals, unsigned long long train_base,
+                                 unsigned long long* out, void* ws, size_t ws_bytes, int sm_count, int variant,
+                                 cudaStream_t stream, const ExchangeArgs* exchange)
+{
+    return resident_of(qbits, nq, q_stride, tprep, nt, train_base, out, ws, ws_bytes, sm_count, variant, stream, exchange,
+                       &runs, totals.tiles);
 }
 
 int launch_tc_knn1_candidates(const KnnProblem& p, const int* list, const int* count, unsigned long long* out, void* ws,
@@ -1269,6 +1389,39 @@ void describe_tc_launch(long long nq, long long nt, int batch, int sm_count, int
 {
     if (variant == HM_VARIANT_F4) describe_of<CoreF4>(nq, nt, batch, sm_count, top1, buf, n);
     else                          describe_of<CoreI8>(nq, nt, batch, sm_count, top1, buf, n);
+}
+
+template <class C>
+static void describe_runs_of(long long nq, const long long* runs4, int n_runs, long long tiles, int sm_count, char* buf,
+                             size_t n, long long* pieces)
+{
+    const TcPlan pl = plan_tc<C>(nq, tiles * C::kTileN, 1, sm_count);
+    if (buf && n) {
+        snprintf(buf, n, "hm_%s_knn2_runs%s_kernel grid=(%lld,%d,1) cluster=%d tiles_per_cta=%d run_tiles=%lld",
+                 C::kScales ? "f4" : "i8", pl.splits > 1 ? "_floor" : "", pl.qblocks, pl.splits, pl.cluster,
+                 pl.tiles_per_split, tiles);
+    }
+    if (!pieces) return;
+    for (int s = 0; s < pl.splits; ++s) {
+        const long long v0 = (long long)s * pl.tiles_per_split, v1 = min(v0 + pl.tiles_per_split, tiles);
+        RunCursor cur;
+        cur.seek(runs4, n_runs, v0);
+        for (long long v = v0; v < v1; ++v) {
+            long long* p = pieces + 4 * v;
+            p[0] = s;
+            p[1] = cur.tile;
+            p[2] = max((long long)cur.tile * kRowBlock, (long long)cur.lo);
+            p[3] = min((long long)(cur.tile + 1) * kRowBlock, (long long)cur.hi);
+            if (v + 1 < v1) cur.next(runs4);
+        }
+    }
+}
+
+void describe_tc_runs(long long nq, const long long* runs_host4, int n_runs, long long tiles, int sm_count, int variant,
+                      char* buf, size_t n, long long* pieces)
+{
+    if (variant == HM_VARIANT_F4) describe_runs_of<CoreF4>(nq, runs_host4, n_runs, tiles, sm_count, buf, n, pieces);
+    else                          describe_runs_of<CoreI8>(nq, runs_host4, n_runs, tiles, sm_count, buf, n, pieces);
 }
 
 int launch_tc_knn2(const KnnProblem& p, unsigned long long* out, void* ws, size_t ws_bytes, int sm_count, int variant,

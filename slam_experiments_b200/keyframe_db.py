@@ -48,6 +48,48 @@ def shard_ranges(sizes: Sequence[int], world_size: int) -> List[Tuple[int, int, 
     return out
 
 
+def selection_mask(keyframes, n_keyframes: int) -> np.ndarray:
+    """A keyframe selection as a bool mask ``[n_keyframes]``.
+
+    ``keyframes`` is a 1-D bool array of length ``n_keyframes`` or a 1-D sequence of integer ``imgIdx`` values (a set:
+    order and duplicates do not matter; an empty sequence selects nothing).  Anything else raises ``MatcherError``."""
+    if isinstance(keyframes, (list, tuple)) and len(keyframes) == 0:
+        return np.zeros(n_keyframes, bool)
+    try:
+        a = np.asarray(keyframes)
+    except Exception as e:
+        raise MatcherError(f"keyframes: not an array ({e})") from None
+    if a.ndim != 1:
+        raise MatcherError("keyframes: expected a 1-D bool mask or a 1-D sequence of imgIdx values")
+    if a.dtype == np.bool_:
+        if a.shape[0] != n_keyframes:
+            raise MatcherError(f"keyframes: bool mask of length {a.shape[0]}, the database has {n_keyframes} keyframes")
+        return a.copy()
+    if a.dtype.kind not in "iu":
+        raise MatcherError(f"keyframes: expected bool or integer values, got {a.dtype}")
+    if a.size and (int(a.min()) < 0 or int(a.max()) >= n_keyframes):
+        raise MatcherError(f"keyframes: imgIdx outside [0, {n_keyframes})")
+    mask = np.zeros(n_keyframes, bool)
+    mask[a] = True
+    return mask
+
+
+def shard_runs(mask: np.ndarray, starts: np.ndarray, kf_lo: int, kf_hi: int, row_lo: int) -> np.ndarray:
+    """The runs ``int64 [n, 2]`` of shard-local rows ``[lo, hi)`` that the selected keyframes of ``[kf_lo, kf_hi)``
+    hold: maximal ranges of rows of consecutive selected keyframes (keyframes without rows hold none), ascending and
+    disjoint.  O(keyframes of the shard)."""
+    sel = np.flatnonzero(mask[kf_lo:kf_hi]) + kf_lo
+    lo, hi = starts[sel], starts[sel + 1]
+    keep = hi > lo
+    lo, hi = lo[keep], hi[keep]
+    if lo.size == 0:
+        return np.empty((0, 2), np.int64)
+    brk = np.flatnonzero(lo[1:] != hi[:-1]) + 1
+    first = np.concatenate([[0], brk])
+    last = np.concatenate([brk, [lo.size]]) - 1
+    return (np.stack([lo[first], hi[last]], axis=1) - row_lo).astype(np.int64)
+
+
 class NativeOps:
     """Device operations of the sharded path: the C ABI kernels + torch.distributed."""
 
@@ -122,6 +164,37 @@ class NativeOps:
             # resident prepared database, packed query: one launch with the f4 core (query expanded in-kernel)
             return nat.knn2_keys_resident(query, shard["prepared"], shard["nt"], train_base, variant=shard["tc"])
         return nat.knn2_keys(query, shard["bits"], train_base=train_base, variant=self.variant)
+
+    # ---- selected keyframes: the shard's runs of selected rows (keyframe_db.shard_runs), never empty here ----
+    def _runs_dev(self, runs: np.ndarray) -> torch.Tensor:
+        """The run table (``_native.run_table``) on the device, through the pinned staging: 32 bytes per run, the
+        row size the staging buffers are built for."""
+        table = nat.run_table(runs)
+        with nat.on_device(self.device):
+            return self._staging.to_device("runs", table.view(np.uint8), self.device).view(torch.int64)
+
+    def local_knn2_runs(self, query: torch.Tensor, shard, train_base: int, runs: np.ndarray) -> torch.Tensor:
+        """Local top-2 over the runs: the tensor-core kernel walks them in place over a prepared image; packed bits are
+        gathered (selected rows only) and searched with ``hm_knn2``."""
+        runs_dev = self._runs_dev(runs)
+        if shard["prepared"] is not None:
+            return nat.knn2_keys_resident_runs(query, shard["prepared"], shard["nt"], runs, runs_dev, train_base,
+                                               variant=shard["tc"])
+        return nat.knn2_keys_runs(query, shard["bits"], runs, runs_dev, train_base, variant=self.variant)
+
+    def local_knn2_runs_exchange(self, query: torch.Tensor, shard, train_base: int, runs: np.ndarray,
+                                 group) -> torch.Tensor:
+        """Local top-2 over the runs + exchange + merge.  Takes the same branch as :meth:`gather_merge` (which a rank
+        without selected rows calls instead): both depend only on ``_xch`` and the query size, and both advance the
+        epoch once."""
+        x = getattr(self, "_xch", None)
+        nq = query.shape[0]
+        if x is None or not (0 < nq <= x["max_rows"]) or shard["prepared"] is None:
+            return self.gather_merge(self.local_knn2_runs(query, shard, train_base, runs), group)
+        x["epoch"] += 1
+        return nat.knn2_keys_resident_runs(query, shard["prepared"], shard["nt"], runs, self._runs_dev(runs), train_base,
+                                           variant=shard["tc"],
+                                           exchange=(x["world"], x["rank"], x["ptrs"], x["max_rows"], x["epoch"]))
 
     def launches_per_step(self, shard, world: int, exchange_mode: str) -> int:
         """Kernels of THIS library launched per ``knn2_keys_device`` call (bench.py's ``gpu_launches``; the ncu launch
@@ -324,9 +397,36 @@ class ShardedKeyframeDatabase:
             self.row_hi += a.shape[0]
         return img
 
+    # ---- selected keyframes ------------------------------------------------------------------------
+    def _selection(self, keyframes):
+        """Validate a ``keyframes=`` argument (before any device work): this rank's runs and the selected rows of the
+        whole database."""
+        mask = selection_mask(keyframes, len(self.sizes))
+        return shard_runs(mask, self.starts, self.kf_lo, self.kf_hi, self.row_lo), int(self.sizes[mask].sum())
+
+    def _knn2_keys_runs(self, query_dev: torch.Tensor, runs: np.ndarray) -> torch.Tensor:
+        """Global top-2 keys over this rank's runs and every other rank's.  A rank without selected rows (or a batch
+        without rows) contributes all-``NO_MATCH`` keys without a k-NN launch but still takes the same exchange as every
+        other rank: which exchange runs depends only on the exchange mode and the query size, both replicated."""
+        nq = query_dev.shape[0]
+        if runs.shape[0] and nq:
+            if self.world_size > 1 and self.exchange_mode == "fused":
+                return self.ops.local_knn2_runs_exchange(query_dev, self.shard, self.row_lo, runs, self.group)
+            local = self.ops.local_knn2_runs(query_dev, self.shard, self.row_lo, runs)
+        else:
+            local = torch.full((nq, 2), -1, dtype=torch.int64, device=query_dev.device)     # HM_NO_MATCH
+        if self.world_size == 1:
+            return local
+        if self.exchange_mode == "fused":
+            return self.ops.gather_merge(local, self.group)
+        return self.ops.merge(self.ops.all_gather(local, self.group))
+
     # ---- device-level API ---------------------------------------------------------------------
-    def knn2_keys_device(self, query_dev: torch.Tensor) -> torch.Tensor:
-        """Global top-2 keys ``[Nq, 2]`` (identical on every rank)."""
+    def knn2_keys_device(self, query_dev: torch.Tensor, keyframes=None) -> torch.Tensor:
+        """Global top-2 keys ``[Nq, 2]`` (identical on every rank).  ``keyframes``: search only these keyframes (a bool
+        mask over ``imgIdx`` or a sequence of ``imgIdx``; every rank passes the same); trainIdx stay global rows."""
+        if keyframes is not None:
+            return self._knn2_keys_runs(query_dev, self._selection(keyframes)[0])
         if self.world_size > 1 and self.exchange_mode == "fused":
             return self.ops.local_knn2_exchange(query_dev, self.shard, self.row_lo, self.group)
         local = self.ops.local_knn2(query_dev, self.shard, self.row_lo)
@@ -336,10 +436,13 @@ class ShardedKeyframeDatabase:
         return self.ops.merge(gathered)
 
     # ---- host-level API -----------------------------------------------------------------------
-    def knn_tensors(self, query: np.ndarray, k: int = 2, while_running=None):
-        """``(imgIdx, trainIdx, distance)`` each ``[Nq, k']``: cv2's collection result as arrays."""
+    def knn_tensors(self, query: np.ndarray, k: int = 2, while_running=None, *, keyframes=None):
+        """``(imgIdx, trainIdx, distance)`` each ``[Nq, k']``: cv2's collection result as arrays.  With ``keyframes``
+        the result over the sub-collection of the selected keyframes, ``imgIdx`` still indexing the whole database
+        (``k' = min(k, selected rows)``)."""
         if k not in (1, 2):
             raise MatcherError("only k in {1, 2} is supported on the B200 path")
+        runs = self._selection(keyframes)[0] if keyframes is not None else None
         q = np.asarray(query)
         if q.size == 0:
             e = np.empty((0, 0), np.int32)
@@ -347,10 +450,11 @@ class ShardedKeyframeDatabase:
         if q.dtype != np.uint8 or q.ndim != 2 or q.shape[1] != nat.DESC_BYTES:
             raise MatcherError("query: expected uint8 [N, 32] descriptors")
         token = None
-        if hasattr(self.ops, "host_query_begin") and (self.world_size == 1 or self.exchange_mode == "fused"):
+        if runs is None and hasattr(self.ops, "host_query_begin") and (self.world_size == 1 or self.exchange_mode == "fused"):
             token = self.ops.host_query_begin(q, self.shard, self.row_lo, self.world_size)
         if token is None:
-            keys_dev = self.knn2_keys_device(self.ops.upload(q))  # enqueued, not finished
+            qd = self.ops.upload(q)
+            keys_dev = self._knn2_keys_runs(qd, runs) if runs is not None else self.knn2_keys_device(qd)  # enqueued
         if while_running is not None:
             while_running()                                       # host work that overlaps the kernels
         keys = self.ops.host_query_end(token) if token is not None else self.ops.to_host(keys_dev)
@@ -361,7 +465,22 @@ class ShardedKeyframeDatabase:
         return img, local, dist
 
     # ---- ratio test + mutual check over the whole database ---------------------------------------------
-    def match_device(self, query_dev: torch.Tensor, *, ratio: Optional[float] = None, cross_check: bool = False):
+    def _match_device(self, query_dev: torch.Tensor, ratio: Optional[float], cross_check: bool, runs):
+        nq = query_dev.shape[0]
+        if not nq:
+            keys = torch.empty((0, 2), dtype=torch.int64, device=query_dev.device)
+        else:
+            keys = self._knn2_keys_runs(query_dev, runs) if runs is not None else self.knn2_keys_device(query_dev)
+        flags = None
+        if cross_check:
+            # the best row of a kept query lies in the selection, so the swapped side needs none
+            flags = self.ops.mutual_flags(keys, query_dev, self.shard, self.row_lo, ratio)
+            if self.world_size > 1:
+                flags = self.ops.all_reduce_max(flags, self.group)
+        return self.ops.filter_matches(keys, flags, ratio)
+
+    def match_device(self, query_dev: torch.Tensor, *, ratio: Optional[float] = None, cross_check: bool = False,
+                     keyframes=None):
         """knnMatch k=2 over the whole database, then Lowe's ratio test and the database-wide mutual check.
 
         Returns device tensors ``(q, t, d, count)``: ``q / t / d [Nq] int32`` hold queryIdx, GLOBAL database row and
@@ -369,47 +488,47 @@ class ShardedKeyframeDatabase:
         ``ratio`` is None or its two nearest rows satisfy ``d1 < ratio * d2`` (float64; a database of fewer than two rows
         drops every query), and -- with ``cross_check`` -- it is the lowest-index nearest query of its best row among
         the ``Nq`` queries of the batch.  Every rank calls it with the same arguments and gets the same list; with
-        ``world_size > 1`` and ``cross_check`` there is one MAX all-reduce over ``Nq`` bytes on the process group."""
-        nq = query_dev.shape[0]
-        keys = self.knn2_keys_device(query_dev) if nq else torch.empty((0, 2), dtype=torch.int64, device=query_dev.device)
-        flags = None
-        if cross_check:
-            flags = self.ops.mutual_flags(keys, query_dev, self.shard, self.row_lo, ratio)
-            if self.world_size > 1:
-                flags = self.ops.all_reduce_max(flags, self.group)
-        return self.ops.filter_matches(keys, flags, ratio)
+        ``world_size > 1`` and ``cross_check`` there is one MAX all-reduce over ``Nq`` bytes on the process group.
+        ``keyframes``: the same over the sub-collection of the selected keyframes (the top-2 inside the selection)."""
+        runs = self._selection(keyframes)[0] if keyframes is not None else None
+        return self._match_device(query_dev, ratio, cross_check, runs)
 
-    def match_tensors(self, query, *, ratio: Optional[float] = None, cross_check: bool = False):
+    def match_tensors(self, query, *, ratio: Optional[float] = None, cross_check: bool = False, keyframes=None):
         """``(queryIdx, imgIdx, trainIdx, distance)`` int32 arrays of :meth:`match_device`, ordered by queryIdx;
         ``(imgIdx, trainIdx)`` locate the best row in the keyframe collection as :meth:`knn_tensors` does."""
+        runs = self._selection(keyframes)[0] if keyframes is not None else None
         q = np.asarray(query)
         if q.size == 0:
             q = np.empty((0, nat.DESC_BYTES), np.uint8)
         if q.dtype != np.uint8 or q.ndim != 2 or q.shape[1] != nat.DESC_BYTES:
             raise MatcherError("query: expected uint8 [N, 32] descriptors")
-        oq, ot, od, cnt = self.match_device(self.ops.upload(q), ratio=ratio, cross_check=cross_check)
+        oq, ot, od, cnt = self._match_device(self.ops.upload(q), ratio, cross_check, runs)
         host = self.ops.to_host(torch.cat([cnt.view(1), oq.view(-1), ot.view(-1), od.view(-1)]))   # one D2H
         n, nq = int(host[0]), q.shape[0]
         qi, gidx, d = host[1:1 + n], host[1 + nq:1 + nq + n], host[1 + 2 * nq:1 + 2 * nq + n]
         img, local = nat.locate_rows(self.starts, gidx.astype(np.int64))
         return qi.astype(np.int32), img, local, d.astype(np.int32)
 
-    def match(self, query, *, ratio: Optional[float] = None, cross_check: bool = False) -> tuple:
+    def match(self, query, *, ratio: Optional[float] = None, cross_check: bool = False, keyframes=None) -> tuple:
         """The kept matches of :meth:`match_tensors` as a tuple of ``cv2.DMatch`` (``imgIdx`` = keyframe index)."""
-        qi, img, local, d = self.match_tensors(query, ratio=ratio, cross_check=cross_check)
+        qi, img, local, d = self.match_tensors(query, ratio=ratio, cross_check=cross_check, keyframes=keyframes)
         return tuple(_build_dmatches(qi, local, d, img))
 
-    def knnMatch(self, queryDescriptors, k: int = 2) -> tuple:
-        """cv2 ``bf.knnMatch(query, k)`` over the whole (sharded) collection."""
+    def knnMatch(self, queryDescriptors, k: int = 2, *, keyframes=None) -> tuple:
+        """cv2 ``bf.knnMatch(query, k)`` over the whole (sharded) collection; with ``keyframes`` over the sub-collection
+        of the selected keyframes (cv2's result for that collection, ``imgIdx`` mapped back to the whole database;
+        ``Nq`` empty tuples when the selection holds no row)."""
         # the result has nq * min(k, rows in the collection) entries whatever the distances turn out to be, so the DMatch
         # objects are allocated while the kernels run and only filled in afterwards
         q = np.asarray(queryDescriptors)
-        kk_known = min(k, int(self.starts[-1])) if k in (1, 2) else 0
+        rows = int(self.starts[-1]) if keyframes is None else self._selection(keyframes)[1]
+        kk_known = min(k, rows) if k in (1, 2) else 0
         pre = []
         if q.ndim == 2 and kk_known > 0:
-            img, local, dist = self.knn_tensors(q, k, while_running=lambda: pre.append(_prealloc_dmatches(q.shape[0] * kk_known, kk_known)))
+            img, local, dist = self.knn_tensors(q, k, while_running=lambda: pre.append(_prealloc_dmatches(q.shape[0] * kk_known, kk_known)),
+                                                keyframes=keyframes)
         else:
-            img, local, dist = self.knn_tensors(queryDescriptors, k)
+            img, local, dist = self.knn_tensors(queryDescriptors, k, keyframes=keyframes)
         nq, kk = img.shape
         if kk == 0:
             return tuple(() for _ in range(nq))
