@@ -65,7 +65,8 @@ typedef enum hm_status {
     HM_OK = 0,
     HM_ERR_INVALID_ARGUMENT = -1, /* cv2 raises cv2.error(-215) for these (batch_distance.cpp:274,282) */
     HM_ERR_CUDA = -2,             /* a CUDA runtime call failed; see hm_last_error() */
-    HM_ERR_WORKSPACE = -3,        /* workspace pointer NULL or smaller than hm_workspace_bytes() */
+    HM_ERR_WORKSPACE = -3,        /* workspace pointer NULL or smaller than its sizing function reports
+                                     (hm_db_mutual_flags: also when not 256-byte aligned) */
     HM_ERR_UNSUPPORTED = -4,      /* shape / variant outside the supported domain */
     HM_ERR_NO_DEVICE = -5         /* no sm_100 device visible: there is NO CPU fallback */
 } hm_status;
@@ -258,7 +259,9 @@ HM_API int hm_filter_matches(const uint64_t* fwd_keys, int64_t nq, const uint64_
  * database-wide answer.  Work is a top-1 k-NN of at most nq gathered shard rows against the nq queries; with the
  * kind::mxf4 core (HM_VARIANT_F4, or AUTO when it resolves to it for nq x nq) only the rows this shard owns are
  * computed, the count of which stays on the device.  Nothing is proportional to the database size: the workspace is
- * hm_db_mutual_workspace_bytes(nq, variant).  flags: HM_FLAG_RATIO and HM_FLAG_MUTUAL only.
+ * hm_db_mutual_workspace_bytes(nq, variant).  flags: HM_FLAG_RATIO and HM_FLAG_MUTUAL only.  Unlike every other
+ * workspace, this one must be 256-byte aligned (the base of a cudaMalloc or torch allocation is): a workspace that is
+ * NULL, smaller, or not 256-byte aligned is HM_ERR_WORKSPACE.
  *
  * hm_db_filter: ratio test (HM_FLAG_RATIO) and mutual check (HM_FLAG_MUTUAL: keep q iff mutual_flags[q] != 0) on the
  * global keys, then the ordered compaction: out_q / out_t / out_d[nq] (queryIdx, global row, distance) ordered by

@@ -28,6 +28,7 @@ FLAG_RATIO, FLAG_MUTUAL, FLAG_DIST_THRESHOLD = 1, 2, 4
 NO_MATCH = 0xFFFFFFFFFFFFFFFF
 DESC_BYTES = 32
 PREPARED_ROW_BYTES = {VARIANT_I8: 256, VARIANT_F4: 128}
+PREPARED_PAD_ROWS = 256         # HM_PREPARED_TILE_ROWS: prepared images are padded to whole blocks of this many rows
 
 # every symbol include/hm_matcher.h declares (tests check the library exports all of them)
 EXPORTS = (

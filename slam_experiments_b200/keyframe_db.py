@@ -125,7 +125,7 @@ class NativeOps:
 
     def append_rows(self, shard, rows: np.ndarray):
         """Grow the resident shard by ``rows`` (a new keyframe): amortised-doubling device buffers, one
-        H2D of the new rows, and re-expansion of the touched 128-row blocks only."""
+        H2D of the new rows, and re-expansion of the touched 256-row blocks only."""
         n = rows.shape[0]
         if n == 0:
             return shard
@@ -152,7 +152,10 @@ class NativeOps:
                                        dtype=torch.uint8, device=self.device)
                     shard["pbuf"] = pbuf
                 elif shard["prepared"] is not None:
-                    first = (nt // 128) * 128                 # the partially filled block and everything after it
+                    # the partially filled block and everything after it.  hm_prepare pads to whole 256-row blocks, so
+                    # starting on a 256-row boundary makes the rewritten rows end exactly at the grown image's padded
+                    # end: every padding row of the image is rewritten, none keeps what the buffer held before.
+                    first = (nt // nat.PREPARED_PAD_ROWS) * nat.PREPARED_PAD_ROWS
                 nat.prepare(buf[first:new_nt], out=pbuf[first * row_bytes:], variant=tc)
                 shard["prepared"] = pbuf
                 shard["tc"] = tc
