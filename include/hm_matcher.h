@@ -355,6 +355,9 @@ HM_API int hm_frame_put(hm_context* ctx, int slot, const uint8_t* desc_host, int
  *      (oracle/orb_oracle.py states every step; results are bit-identical to cv2 4.13 for the same keypoints). */
 #define HM_ORB_MAX_LEVELS 16
 #define HM_ORB_BORDER 32
+/* A geometry (rows, cols, n_levels) is accepted when 1 <= n_levels <= HM_ORB_MAX_LEVELS, each side is at most 16384 and
+ * every level 0 .. n_levels-1 is more than HM_ORB_BORDER pixels on both sides (the reflected frame fits inside it).
+ * Otherwise hm_orb_workspace_bytes returns 0 and the calls below return HM_ERR_INVALID_ARGUMENT. */
 HM_API size_t hm_orb_workspace_bytes(int rows, int cols, int n_levels);
 /* size and 1 / scale of pyramid level `level` (host arithmetic, no device needed) */
 HM_API int hm_orb_level_geometry(int rows, int cols, int level, int* out_rows, int* out_cols, float* out_inv_scale);
@@ -365,7 +368,8 @@ HM_API int hm_orb_build_pyramid(const uint8_t* image, int rows, int cols, int64_
                                 void* workspace, size_t workspace_bytes, void* stream);
 /* n keypoints: kp_xy = KeyPoint.pt (level-0 pixels, float pairs, 8-byte aligned), kp_cs = hm_orb_angles_to_cs of
  * KeyPoint.angle, kp_octave = KeyPoint.octave (< n_levels) -> out_desc[n] rows of 32 bytes, `out_stride` bytes apart.
- * `workspace` is the one hm_orb_build_pyramid filled for the same (rows, cols, n_levels). */
+ * `workspace` is the one hm_orb_build_pyramid filled for the same (rows, cols, n_levels).  Octaves are not checked here:
+ * one outside 0 .. n_levels-1 is clamped to that range (hm_frame_put_orb rejects them). */
 HM_API int hm_orb_describe(const void* workspace, int rows, int cols, int n_levels, const float* kp_xy, const float* kp_cs,
                            const int32_t* kp_octave, int64_t n, uint8_t* out_desc, int64_t out_stride, void* stream);
 /* Host image + keypoints -> descriptors written straight into frame slot `slot` (they never visit the host unless

@@ -43,11 +43,13 @@ struct OrbGeometry {
     OrbLevel lv[kMaxLevels];
 };
 
-// Host arithmetic, identical to ORB_Impl::detectAndCompute's layer set-up: getScale() is (float)pow((double)1.2f, level)
+// Host arithmetic, identical to ORB_Impl::detectAndCompute's layer set-up: getScale() is (float)pow((double)1.2f, level).
+// Accepted: each side of level 0 at most 16384, 1 .. 16 levels, and every level more than 32 pixels on both sides
+// (checked in the loop; level 0 is the image itself).
 int orb_geometry(int rows, int cols, int n_levels, OrbGeometry* g)
 {
-    if (rows < 2 * kBorder || cols < 2 * kBorder || rows > 16384 || cols > 16384 || n_levels < 1 || n_levels > kMaxLevels) {
-        set_error("hm_orb: image %d x %d with %d levels is out of range (each side 64 .. 16384, levels 1 .. %d)", rows, cols,
+    if (rows > 16384 || cols > 16384 || n_levels < 1 || n_levels > kMaxLevels) {
+        set_error("hm_orb: image %d x %d with %d levels is out of range (each side at most 16384, levels 1 .. %d)", rows, cols,
                   n_levels, kMaxLevels);
         return HM_ERR_INVALID_ARGUMENT;
     }
@@ -62,8 +64,8 @@ int orb_geometry(int rows, int cols, int n_levels, OrbGeometry* g)
         L.rows = (int)lrintf((float)rows * L.inv_scale);
         L.cols = (int)lrintf((float)cols * L.inv_scale);
         if (L.rows <= kBorder || L.cols <= kBorder) {     // the reflected frame must fit inside the level
-            set_error("hm_orb: level %d of a %d x %d image is %d x %d, smaller than the %d-pixel frame", l, rows, cols, L.rows,
-                      L.cols, kBorder);
+            set_error("hm_orb: level %d of a %d x %d image is %d x %d; every level must be more than %d pixels on both sides "
+                      "(the reflected frame)", l, rows, cols, L.rows, L.cols, kBorder);
             return HM_ERR_INVALID_ARGUMENT;
         }
         L.stride = (L.cols + 2 * kBorder + 15) / 16 * 16;

@@ -44,11 +44,15 @@ def keypoint_arrays(keypoints: Sequence[KeyPoint]):
     return xy, ang, octv
 
 
-class OrbFeatureDetector(FeatureDetector):
-    """`feature_detectors.py:18-26`, descriptors on the device.  ``n_levels`` is cv2's default (8): the reference
-    never changes it."""
+def pyramid_levels(octaves: np.ndarray) -> int:
+    """Levels of the pyramid the descriptors of these keypoints need: ``max(octave) + 1``, as ``cv2.ORB.compute`` builds
+    it for keypoints passed in (1 for none).  On a small image cv2's detector stops short of its 8 levels, and the
+    levels it never reached may be too small to hold the 32-pixel frame."""
+    return int(octaves.max()) + 1 if octaves.size else 1
 
-    N_LEVELS = 8
+
+class OrbFeatureDetector(FeatureDetector):
+    """`feature_detectors.py:18-26`, descriptors on the device."""
 
     def __init__(self, n_features: int = 500, device=None) -> None:
         self.orb = ORB.create(nfeatures=n_features)
@@ -68,12 +72,13 @@ class OrbFeatureDetector(FeatureDetector):
     def compute_device(self, img: np.ndarray, keypoints: Sequence[KeyPoint]) -> torch.Tensor:
         """The same descriptors as a ``[n, 32] uint8`` CUDA tensor (no D2H)."""
         xy, ang, octv = keypoint_arrays(keypoints)
+        n_levels = pyramid_levels(octv)
         with nat.on_device(self.device):
             image = torch.from_numpy(np.ascontiguousarray(img)).to(self.device)
-            self._workspace = nat.orb_build_pyramid(image, self.N_LEVELS, self._workspace)
+            self._workspace = nat.orb_build_pyramid(image, n_levels, self._workspace)
             pack = torch.from_numpy(np.concatenate([xy.reshape(-1), nat.orb_angles_to_cs(ang).reshape(-1)])).to(self.device)
             n = xy.shape[0]
-            return nat.orb_describe(self._workspace, img.shape[:2], self.N_LEVELS, pack[:2 * n].view(n, 2),
+            return nat.orb_describe(self._workspace, img.shape[:2], n_levels, pack[:2 * n].view(n, 2),
                                     pack[2 * n:].view(n, 2), torch.from_numpy(octv).to(self.device))
 
     def detect_and_compute(self, img: np.ndarray, mask: np.ndarray = None) -> tuple[Sequence[KeyPoint], np.ndarray]:
@@ -86,5 +91,5 @@ class OrbFeatureDetector(FeatureDetector):
         `/root/reference/primitives.py`) are stored with the frame so that matched points can be gathered on the
         device."""
         keypoints = self.orb.detect(img, mask)
-        store.put_image(frame_id, img, keypoints, n_levels=self.N_LEVELS, with_positions=with_positions)
+        store.put_image(frame_id, img, keypoints, with_positions=with_positions)
         return keypoints

@@ -155,16 +155,19 @@ class FrameDescriptorStore:
             del self._frames[frame_id]
             self._points.pop(frame_id, None)
 
-    def put_image(self, frame_id, image: np.ndarray, keypoints, n_levels: int = 8, with_positions: bool = True,
+    def put_image(self, frame_id, image: np.ndarray, keypoints, n_levels: Optional[int] = None, with_positions: bool = True,
                   want_descriptors: bool = False):
         """Store a frame from its IMAGE and cv2 keypoints: the ORB descriptors are computed on the device
         (``hm_frame_put_orb``, SURVEY.md 8f rank 3) and written into the frame's slot without visiting the host.
+        ``n_levels=None`` builds ``max(octave) + 1`` pyramid levels, as ``cv2.ORB.compute`` does for given keypoints.
         Returns the descriptors only when ``want_descriptors``."""
-        from .feature_detectors import keypoint_arrays
+        from .feature_detectors import keypoint_arrays, pyramid_levels
         if self._ctx is None:
             with nat.on_device(self.device):
                 self._ctx = nat.HostContext()
         xy, ang, octv = keypoint_arrays(keypoints)
+        if n_levels is None:
+            n_levels = pyramid_levels(octv)
         pos = xy.astype(np.int32) if with_positions else None      # Feature.position: int() of the keypoint coordinates
         if frame_id in self._slots:
             slot = self._slots.pop(frame_id)[0]

@@ -94,15 +94,20 @@ def test_oracle_describe_equals_cv2_live():
         assert np.array_equal(desc2, desc) and len(kps2) == len(kps)
 
 
-def test_library_geometry_and_angles_without_a_device():
+def test_library_frame_rule_geometry_and_angles_without_a_device():
+    """Level sizes and scales, the per-level frame rule (a level only has to be more than 32 pixels, so a 40-pixel
+    side is accepted and a 32-pixel one is not), and the (cos, sin) arithmetic, all on the host."""
     hm_build.build()
     for h, w in ((480, 640), (480, 752), (333, 517), (1920, 2560), (1080, 1920)):
         for lv in range(8):
             r, c, inv = nat.orb_level_geometry(h, w, lv)
             assert (r, c) == oo.level_size(h, w, lv)
             assert np.float32(inv) == np.float32(1.0) / oo.level_scale(lv)
+    assert nat.orb_level_geometry(40, 640, 0)[:2] == (40, 640)     # a level only has to hold the 32-pixel frame
     with pytest.raises(nat.NativeError):
-        nat.orb_level_geometry(40, 640, 0)
+        nat.orb_level_geometry(32, 640, 0)
+    with pytest.raises(nat.NativeError):
+        nat.orb_level_geometry(640, 32, 0)
     ang = np.concatenate([np.random.default_rng(0).random(200000).astype(np.float32) * np.float32(360), np.arange(0, 360, 0.5, dtype=np.float32)])
     rad = ang * np.float32(math.pi / np.float32(180.0))
     ref = np.stack([np.cos(rad.astype(np.float64)).astype(np.float32), np.sin(rad.astype(np.float64)).astype(np.float32)], 1)
